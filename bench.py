@@ -2,6 +2,7 @@
 """bench.py — column RK-steps/s of the batched RK45 integrator and time-to-T* (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-tstar] [--no-large-n]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d config 2): the synthetic 4096-column
 Map_Scenario parameter sweep (16 x 16 x 16 lattice over sedimentation rate, b, D0co3), N=200
@@ -29,6 +30,10 @@ the data path, one NCCL all-gather of the end states after the timed steps.
 `cpu_baseline` / `--impl reference`: the reference's own path — SciPy solve_ivp(RK45) driving the
            restated numba RHS (oracle/, kind "port": py-pde is not installable here) — on the
            host cores of the same box, one column per process, bounded sample.
+`--dump-outputs DIR` writes what the headline step returned after the last timed step as DIR/<name>.npy (float64; see
+           dump_outputs), so that two builds run with the same arguments can be compared output for output.
+
+The benchmark writes nothing into the source tree: no bytecode, and numba's cache goes to a temporary directory.
 """
 from __future__ import annotations
 
@@ -38,6 +43,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -298,6 +304,37 @@ def timed_steps(stepper, steps, flush, barrier):
     return a1 - a0, sum(a.elapsed_time(b) for a, b in ev), w0, w1
 
 
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, stepper, rank, world):
+    """What the headline step hands its caller, as float64 .npy files: the column states `y` [B, 5, N], the per-column
+    integrator records `state_*` (t, h_abs, step counts, nfev, status), the event monitors' `event_counts` [B, 7] and
+    `event_times`: the located roots only, min(count, evcap) of them per column and monitor, concatenated in
+    (column, monitor) order (the kernel fills slots from 0 and leaves the rest of the NaN-filled buffer untouched).
+    `column_index` says which columns of this rank's block were written: all of them when they fit
+    DUMP_BUDGET_BYTES with every event slot filled (4096 columns at N=200: 37 MB at most), else a sample drawn
+    with a fixed seed.
+    At N>1 GPUs every rank writes its own block, file names suffixed with _rank<r>."""
+    import numpy as np
+    st = stepper.state()
+    per_column = 8 * (5 * stepper.N + 7 + 7 * stepper.evcap + 7)
+    keep = min(stepper.B, DUMP_BUDGET_BYTES // world // per_column)
+    cols = np.arange(stepper.B)
+    if keep < stepper.B:
+        cols = np.sort(np.random.default_rng(0).choice(stepper.B, keep, replace=False))
+    counts = stepper.d_ec.cpu().numpy()[cols]
+    located = np.arange(stepper.evcap) < np.minimum(counts, stepper.evcap)[..., None]
+    arrays = {"column_index": cols, "y": stepper.d_y.cpu().numpy()[cols],
+              "event_counts": counts, "event_times": stepper.d_et.cpu().numpy()[cols][located]}
+    for field in ("t", "h_abs", "n_accepted", "n_rejected", "nfev", "status"):
+        arrays["state_" + field] = st[field][cols]
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def radau_algorithmic_bytes(n_cells, newton, nlu, njev, steps_attempted):
     """HBM bytes the implicit kernel has to move by construction (DESIGN.md §5): all per-column vectors, Jacobian
     blocks and fp32 records live in a per-column HBM workspace.  V = 5 N doubles (one state-sized vector).
@@ -423,6 +460,8 @@ def run_gpu_arm(args, rank: int, local_rank: int, world: int):
     st = stepper.state()
     kernel_ms = dev_ms / args.steps
     clocks = sampler.summary(w0, w1) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, stepper, rank, world)
 
     # ---- e2e: the host-pointer C-ABI call with pinned host buffers, copies inside the timed region
     h_y = torch.from_numpy(stepper.d_y.cpu().numpy()).pin_memory()
@@ -729,7 +768,14 @@ def main():
     ap.add_argument("--no-cpu-radau", action="store_true", help="skip the SciPy Radau sample beside the implicit sweep")
     ap.add_argument("--no-bdf", action="store_true", help="N=1: skip the BDF sweep to T* (~20 s + its SciPy BDF sample)")
     ap.add_argument("--cpu-t-end", type=float, default=0.03, help="CPU sample: integrate to this fraction of T*")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline step's outputs after the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
+    # the tree may be read-only: no bytecode next to the sources, numba's cache (oracle/, cache=True) elsewhere
+    sys.dont_write_bytecode = True
+    os.environ.setdefault("NUMBA_CACHE_DIR", os.path.join(tempfile.gettempdir(), f"marlpde-bench-numba-{os.getuid()}"))
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

@@ -2,7 +2,8 @@
 the drop-in mirror: same imports, same calls, same tolerances — `integrate_equations` with the default
 `Solver()` (Radau, rtol = atol = 1e-3), final-time fields against the reference's HDF5 fixtures (decoded
 once into tests/golden/fixtures_reference.npz; h5py is not installed here) — plus the HDF5 output layout
-(Evolve_scenario.py:157-178) and the RK45 / SciPy-stepper routes of the same entry point."""
+(Evolve_scenario.py:157-178) and the RK45 / SciPy-stepper routes of the same entry point, the SciPy Radau stepper
+driving the CUDA RHS to T* included."""
 import glob
 import os
 from dataclasses import asdict
@@ -95,6 +96,24 @@ def test_rk45_and_scipy_stepper_routes(fixtures_reference, in_tmp_cwd, monkeypat
     assert covered == pytest.approx(scen["Tstar"] * 0.002)
     c, _, _, _, _ = integrate_equations(asdict(Solver(method="LSODA")) | short, dict(tr), dict(scen))
     assert_allclose(a, c, rtol=0, atol=2e-2)              # LSODA with the reference's lband = uband = 1
+
+
+def test_scipy_radau_stepper_with_cuda_rhs_matches_fixture(fixtures_reference, in_tmp_cwd, monkeypatch):
+    """The reference's own loop to T* (Evolve_scenario.py:104-109): SciPy's Radau with the reference's jac_sparsity
+    (finite-difference Jacobian by column groups) steps scenario A, every RHS evaluation is the CUDA kernel through
+    `eq.fun_numba`; final fields against the reference's fixture at its tolerances."""
+    import marlpde_b200
+
+    def no_device_stepper(*a, **kw):
+        raise AssertionError("MARLPDE_SCIPY_STEPPER=1 must leave the stepping to SciPy")
+    monkeypatch.setattr(marlpde_b200, "integrate_radau_batch", no_device_stepper)
+    monkeypatch.setenv("MARLPDE_SCIPY_STEPPER", "1")
+    scen = asdict(Map_Scenario()) | {"Phi0": 0.6, "PhiIni": 0.5, "PhiNR": 0.6}
+    solver = asdict(Solver())
+    assert solver["method"] == "Radau" and solver["jac_sparsity"] is not None
+    last_field_sol, covered_time, _, _, _ = integrate_equations(solver, asdict(Tracker()), scen)
+    assert_allclose(last_field_sol, fixtures_reference["scenario_A"][-1], rtol=0.1, atol=0.01)
+    assert covered_time == scen["Tstar"]
 
 
 @pytest.mark.parametrize("n_cells", [16, 1000])

@@ -106,15 +106,30 @@ def test_cabi_exports_every_declared_symbol():
     assert L.marlpde_rk45_columns_per_cta(641) == 0 and L.marlpde_rk45_columns_per_cta(16) == 0
 
 
+_NO_DEVICE_CHECK = """
+import pytest
+import lheureux_oracle as oracle
+import marlpde_b200 as mb
+from marlpde_b200 import _cabi
+assert _cabi.lib().marlpde_device_count() == 0
+pde = oracle.default_scenario()
+with pytest.raises(_cabi.MarlpdeError, match="no CUDA device"):
+    mb.rhs_batch(mb.initial_state(pde), mb.derive_column_params(pde))
+with pytest.raises(_cabi.MarlpdeError, match="no CUDA device"):
+    mb.integrate_rk45_batch(mb.initial_state(pde), mb.derive_column_params(pde), t_span=(0, 1e-4))
+"""
+
+
 def test_no_device_fails_loudly():
-    """The product has no CPU fallback: on a box without a GPU compute calls must raise."""
-    if _cabi.lib().marlpde_device_count() > 0:
-        pytest.skip("a CUDA device is present")
-    pde = oracle.default_scenario()
-    with pytest.raises(_cabi.MarlpdeError, match="no CUDA device"):
-        mb.rhs_batch(mb.initial_state(pde), mb.derive_column_params(pde))
-    with pytest.raises(_cabi.MarlpdeError, match="no CUDA device"):
-        mb.integrate_rk45_batch(mb.initial_state(pde), mb.derive_column_params(pde), t_span=(0, 1e-4))
+    """The product has no CPU fallback: on a box without a GPU compute calls must raise.  Runs in a child process
+    with every device hidden (CUDA_VISIBLE_DEVICES=""), so it checks the same on a machine that has one."""
+    import subprocess
+    import sys
+    path = [os.path.join(ROOT, "integrating-diagenetic-equations-using-python_b200"), os.path.join(ROOT, "oracle"),
+            os.environ.get("PYTHONPATH", "")]
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="", PYTHONPATH=os.pathsep.join(p for p in path if p))
+    done = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHECK], env=env, capture_output=True, text=True, timeout=300)
+    assert done.returncode == 0, done.stderr[-2000:]
 
 
 def test_argument_validation_before_any_device_work():
