@@ -14,6 +14,8 @@
  *     call site marlpde/Evolve_scenario.py:104-109
  *   scipy.integrate.solve_ivp(method="Radau", jac_sparsity=jacobian_sparsity())   marlpde_radau_integrate[_dev]
  *     the reference's default Solver (marlpde/parameters.py:150-199, :213)
+ *   scipy.integrate.solve_ivp(method="BDF" | "LSODA")    marlpde_bdf_integrate[_dev]
+ *   scipy.integrate.solve_ivp(method="RK23" | "DOP853")  marlpde_rk23_integrate[_dev], marlpde_dop853_integrate[_dev]
  *   7 event monitors (LHeureux_model.py:524-593)          event outputs of marlpde_rk45_integrate*
  *   derived constants of __init__ (:31-72, :130-133)      marlpde_column_params (filled by the host
  *                                                          mirror, one struct per sediment column)
@@ -279,6 +281,47 @@ int marlpde_bdf_integrate_async(double* y, const marlpde_column_params* params,
                                 const marlpde_rk45_options* opts, const double* t_eval,
                                 double* snapshots, int32_t* event_counts, double* event_times,
                                 int64_t* stats, int device, void* stream);
+
+/* ---- batched explicit Runge-Kutta integrators: Bogacki-Shampine RK23 and Dormand-Prince DOP853
+ * (replace solve_ivp(method="RK23" | "DOP853") per column — marlpde/parameters.py:213; scipy/integrate/_ivp/rk.py —
+ * step for step: same tableaux, step-size control, error norms and dense output, see csrc/erk_batch.cu) ------------
+ *  Arguments and outputs as for marlpde_bdf_integrate* without the statistics: same options struct (opts->quantum
+ *  must be 0), same column state and status codes; t_eval samples and events use each method's dense output (DOP853:
+ *  the three extra stages are evaluated, and counted in nfev, only in steps that sample t_eval or locate an event).
+ *  The workspace is marlpde_{rk23,dop853}_workspace_bytes(n_columns, n_cells); d_queue is one zeroed int32.  Any
+ *  n_cells >= 3.  A column that stops on the step budget stops after an accepted step and resumes from (t, h_abs, y)
+ *  bit-identically (nfev counts one extra evaluation of f(y) per resume).
+ */
+size_t marlpde_rk23_workspace_bytes(int n_columns, int n_cells);
+int marlpde_rk23_integrate_dev(double* d_y, const marlpde_column_params* d_params,
+                               marlpde_column_state* d_state, int n_columns, int n_cells,
+                               const marlpde_rk45_options* opts, const double* d_t_eval,
+                               double* d_snapshots, int32_t* d_event_counts, double* d_event_times,
+                               void* d_workspace, size_t workspace_bytes, int32_t* d_queue, void* stream);
+int marlpde_rk23_integrate(double* y, const marlpde_column_params* params,
+                           marlpde_column_state* state, int n_columns, int n_cells,
+                           const marlpde_rk45_options* opts, const double* t_eval,
+                           double* snapshots, int32_t* event_counts, double* event_times, int device);
+int marlpde_rk23_integrate_async(double* y, const marlpde_column_params* params,
+                                 marlpde_column_state* state, int n_columns, int n_cells,
+                                 const marlpde_rk45_options* opts, const double* t_eval,
+                                 double* snapshots, int32_t* event_counts, double* event_times,
+                                 int device, void* stream);
+size_t marlpde_dop853_workspace_bytes(int n_columns, int n_cells);
+int marlpde_dop853_integrate_dev(double* d_y, const marlpde_column_params* d_params,
+                                 marlpde_column_state* d_state, int n_columns, int n_cells,
+                                 const marlpde_rk45_options* opts, const double* d_t_eval,
+                                 double* d_snapshots, int32_t* d_event_counts, double* d_event_times,
+                                 void* d_workspace, size_t workspace_bytes, int32_t* d_queue, void* stream);
+int marlpde_dop853_integrate(double* y, const marlpde_column_params* params,
+                             marlpde_column_state* state, int n_columns, int n_cells,
+                             const marlpde_rk45_options* opts, const double* t_eval,
+                             double* snapshots, int32_t* event_counts, double* event_times, int device);
+int marlpde_dop853_integrate_async(double* y, const marlpde_column_params* params,
+                                   marlpde_column_state* state, int n_columns, int n_cells,
+                                   const marlpde_rk45_options* opts, const double* t_eval,
+                                   double* snapshots, int32_t* event_counts, double* event_times,
+                                   int device, void* stream);
 
 /* ---- measurement helper: fp64 FMA peak (TFLOP/s, best of `repeats`) of `device`, the roofline
  * denominator of the fp64-pipe-bound RK45 kernel (no reference counterpart). */

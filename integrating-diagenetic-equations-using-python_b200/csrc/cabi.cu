@@ -13,6 +13,7 @@
 
 #include "../../include/marlpde_b200.h"
 #include "bdf_batch.cuh"
+#include "erk_batch.cuh"
 #include "radau_batch.cuh"
 #include "rk45_persistent.cuh"
 #include "rk45_streaming.cuh"
@@ -655,6 +656,154 @@ int marlpde_bdf_integrate_async(double* y, const marlpde_column_params* params, 
                                 int device, void* stream) {
   return implicit_integrate_host(kBdf, y, params, state, n_columns, n_cells, opts, t_eval, snapshots, event_counts,
                                  event_times, stats, device, (cudaStream_t)stream, false);
+}
+
+// ---- explicit Runge-Kutta integrators (RK23, DOP853): the implicit integrators' buffers and checks, no statistics ----
+static const char* erk_name(marlpde::ErkMethod m) { return m == marlpde::kErkRK23 ? "rk23" : "dop853"; }
+
+static int check_erk_args(marlpde::ErkMethod m, int n_columns, int n_cells, const marlpde_rk45_options* opts) {
+  if (!opts) return fail(MARLPDE_EINVAL, "opts is NULL");
+  if (n_columns < 0) return fail(MARLPDE_EINVAL, "n_columns < 0");
+  if (n_cells < 3) return fail(MARLPDE_EINVAL, "the %s integrator needs n_cells >= 3 (got %d)", erk_name(m), n_cells);
+  if (!(opts->rtol > 0.0) || !(opts->atol >= 0.0)) return fail(MARLPDE_EINVAL, "need rtol > 0, atol >= 0");
+  if (!(opts->max_step > 0.0)) return fail(MARLPDE_EINVAL, "max_step must be positive (use +inf for none)");
+  if (opts->n_eval < 0 || opts->event_capacity < 0) return fail(MARLPDE_EINVAL, "negative n_eval/event_capacity");
+  if (opts->quantum != 0) return fail(MARLPDE_EUNSUPPORTED, "opts->quantum is not used by the %s integrator (pass 0)", erk_name(m));
+  return MARLPDE_OK;
+}
+
+static int erk_integrate_dev(marlpde::ErkMethod m, double* d_y, const marlpde_column_params* d_params,
+                             marlpde_column_state* d_state, int n_columns, int n_cells, const marlpde_rk45_options* opts,
+                             const double* d_t_eval, double* d_snapshots, int32_t* d_event_counts, double* d_event_times,
+                             void* d_workspace, size_t workspace_bytes, int32_t* d_queue, void* stream) {
+  int rc = check_erk_args(m, n_columns, n_cells, opts);
+  if (rc) return rc;
+  if (n_columns == 0) return MARLPDE_OK;
+  if (!d_y || !d_params || !d_state || !d_queue || !d_workspace) return fail(MARLPDE_EINVAL, "NULL device pointer");
+  if (opts->n_eval > 0 && (!d_t_eval || !d_snapshots)) return fail(MARLPDE_EINVAL, "n_eval > 0 needs t_eval and snapshots");
+  if (opts->flags & MARLPDE_FLAG_EVENTS) {
+    if (!d_event_counts) return fail(MARLPDE_EINVAL, "MARLPDE_FLAG_EVENTS needs event_counts");
+    if (opts->event_capacity > 0 && !d_event_times) return fail(MARLPDE_EINVAL, "event_capacity > 0 needs event_times");
+  }
+  const size_t need = marlpde::erk_workspace_bytes(m, n_columns, n_cells);
+  if (workspace_bytes < need) return fail(MARLPDE_EINVAL, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
+  DevProps props;
+  rc = current_props(props);
+  if (rc) return rc;
+  cudaError_t e = marlpde::launch_erk(m, d_y, d_params, d_state, n_columns, n_cells, *opts, d_t_eval, d_snapshots,
+                                      d_event_counts, d_event_times, static_cast<double*>(d_workspace), d_queue,
+                                      props.sm_count, (cudaStream_t)stream);
+  if (e != cudaSuccess) return cuda_fail(e, m == marlpde::kErkRK23 ? "rk23 launch" : "dop853 launch");
+  return MARLPDE_OK;
+}
+
+static int erk_integrate_host(marlpde::ErkMethod m, double* y, const marlpde_column_params* params,
+                              marlpde_column_state* state, int n_columns, int n_cells, const marlpde_rk45_options* opts,
+                              const double* t_eval, double* snapshots, int32_t* event_counts, double* event_times,
+                              int device, cudaStream_t s, bool sync) {
+  int rc = check_erk_args(m, n_columns, n_cells, opts);
+  if (rc) return rc;
+  if (n_columns == 0) return MARLPDE_OK;
+  if (!y || !params || !state) return fail(MARLPDE_EINVAL, "NULL pointer");
+  if (opts->n_eval > 0 && (!t_eval || !snapshots)) return fail(MARLPDE_EINVAL, "n_eval > 0 needs t_eval and snapshots");
+  DeviceScope scope;
+  rc = scope.enter(device);
+  if (rc) return rc;
+  const size_t nb_y = sizeof(double) * 5 * (size_t)n_cells * n_columns;
+  const size_t nb_snap = nb_y * (size_t)opts->n_eval;
+  const size_t nb_p = sizeof(marlpde_column_params) * (size_t)n_columns;
+  const size_t nb_s = sizeof(marlpde_column_state) * (size_t)n_columns;
+  const size_t nb_work = marlpde::erk_workspace_bytes(m, n_columns, n_cells);
+  const size_t nb_ec = sizeof(int32_t) * MARLPDE_NEVENTS * (size_t)n_columns;
+  const size_t nb_et = sizeof(double) * MARLPDE_NEVENTS * (size_t)opts->event_capacity * n_columns;
+  DevBuf dy, dp, ds, dte, dsnap, dq, dw, dec, det;
+  CU(dy.alloc(nb_y, s));
+  CU(dp.alloc(nb_p, s));
+  CU(ds.alloc(nb_s, s));
+  CU(dte.alloc(sizeof(double) * (size_t)opts->n_eval, s));
+  CU(dsnap.alloc(nb_snap, s));
+  CU(dq.alloc(sizeof(int32_t), s));
+  CU(dw.alloc(nb_work, s));
+  CU(dec.alloc(nb_ec, s));
+  CU(det.alloc(nb_et, s));
+  CU(cudaMemcpyAsync(dy.p, y, nb_y, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dp.p, params, nb_p, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(ds.p, state, nb_s, cudaMemcpyHostToDevice, s));
+  if (opts->n_eval) CU(cudaMemcpyAsync(dte.p, t_eval, sizeof(double) * (size_t)opts->n_eval, cudaMemcpyHostToDevice, s));
+  if (snapshots && nb_snap) CU(cudaMemcpyAsync(dsnap.p, snapshots, nb_snap, cudaMemcpyHostToDevice, s));
+  CU(cudaMemsetAsync(dq.p, 0, sizeof(int32_t), s));
+  if (event_counts) CU(cudaMemcpyAsync(dec.p, event_counts, nb_ec, cudaMemcpyHostToDevice, s));
+  else CU(cudaMemsetAsync(dec.p, 0, nb_ec, s));
+  if (event_times && nb_et) CU(cudaMemcpyAsync(det.p, event_times, nb_et, cudaMemcpyHostToDevice, s));
+  marlpde_rk45_options o = *opts;
+  o.flags |= model_flags_of(params, n_columns);
+  rc = erk_integrate_dev(m, dy.as<double>(), dp.as<marlpde_column_params>(), ds.as<marlpde_column_state>(), n_columns,
+                         n_cells, &o, dte.as<double>(), dsnap.as<double>(), dec.as<int32_t>(), det.as<double>(), dw.p,
+                         nb_work, dq.as<int32_t>(), s);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(y, dy.p, nb_y, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(state, ds.p, nb_s, cudaMemcpyDeviceToHost, s));
+  if (snapshots && nb_snap) CU(cudaMemcpyAsync(snapshots, dsnap.p, nb_snap, cudaMemcpyDeviceToHost, s));
+  if (event_counts) CU(cudaMemcpyAsync(event_counts, dec.p, nb_ec, cudaMemcpyDeviceToHost, s));
+  if (event_times && nb_et) CU(cudaMemcpyAsync(event_times, det.p, nb_et, cudaMemcpyDeviceToHost, s));
+  if (sync) CU(cudaStreamSynchronize(s));
+  return MARLPDE_OK;
+}
+
+size_t marlpde_rk23_workspace_bytes(int n_columns, int n_cells) {
+  if (n_columns <= 0 || n_cells <= 0) return 0;
+  return marlpde::erk_workspace_bytes(marlpde::kErkRK23, n_columns, n_cells);
+}
+
+size_t marlpde_dop853_workspace_bytes(int n_columns, int n_cells) {
+  if (n_columns <= 0 || n_cells <= 0) return 0;
+  return marlpde::erk_workspace_bytes(marlpde::kErkDOP853, n_columns, n_cells);
+}
+
+int marlpde_rk23_integrate_dev(double* d_y, const marlpde_column_params* d_params, marlpde_column_state* d_state,
+                               int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* d_t_eval,
+                               double* d_snapshots, int32_t* d_event_counts, double* d_event_times, void* d_workspace,
+                               size_t workspace_bytes, int32_t* d_queue, void* stream) {
+  return erk_integrate_dev(marlpde::kErkRK23, d_y, d_params, d_state, n_columns, n_cells, opts, d_t_eval, d_snapshots,
+                           d_event_counts, d_event_times, d_workspace, workspace_bytes, d_queue, stream);
+}
+
+int marlpde_dop853_integrate_dev(double* d_y, const marlpde_column_params* d_params, marlpde_column_state* d_state,
+                                 int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* d_t_eval,
+                                 double* d_snapshots, int32_t* d_event_counts, double* d_event_times, void* d_workspace,
+                                 size_t workspace_bytes, int32_t* d_queue, void* stream) {
+  return erk_integrate_dev(marlpde::kErkDOP853, d_y, d_params, d_state, n_columns, n_cells, opts, d_t_eval, d_snapshots,
+                           d_event_counts, d_event_times, d_workspace, workspace_bytes, d_queue, stream);
+}
+
+int marlpde_rk23_integrate(double* y, const marlpde_column_params* params, marlpde_column_state* state, int n_columns,
+                           int n_cells, const marlpde_rk45_options* opts, const double* t_eval, double* snapshots,
+                           int32_t* event_counts, double* event_times, int device) {
+  return erk_integrate_host(marlpde::kErkRK23, y, params, state, n_columns, n_cells, opts, t_eval, snapshots,
+                            event_counts, event_times, device, cudaStreamPerThread, true);
+}
+
+int marlpde_dop853_integrate(double* y, const marlpde_column_params* params, marlpde_column_state* state, int n_columns,
+                             int n_cells, const marlpde_rk45_options* opts, const double* t_eval, double* snapshots,
+                             int32_t* event_counts, double* event_times, int device) {
+  return erk_integrate_host(marlpde::kErkDOP853, y, params, state, n_columns, n_cells, opts, t_eval, snapshots,
+                            event_counts, event_times, device, cudaStreamPerThread, true);
+}
+
+int marlpde_rk23_integrate_async(double* y, const marlpde_column_params* params, marlpde_column_state* state,
+                                 int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* t_eval,
+                                 double* snapshots, int32_t* event_counts, double* event_times, int device,
+                                 void* stream) {
+  return erk_integrate_host(marlpde::kErkRK23, y, params, state, n_columns, n_cells, opts, t_eval, snapshots,
+                            event_counts, event_times, device, (cudaStream_t)stream, false);
+}
+
+int marlpde_dop853_integrate_async(double* y, const marlpde_column_params* params, marlpde_column_state* state,
+                                   int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* t_eval,
+                                   double* snapshots, int32_t* event_counts, double* event_times, int device,
+                                   void* stream) {
+  return erk_integrate_host(marlpde::kErkDOP853, y, params, state, n_columns, n_cells, opts, t_eval, snapshots,
+                            event_counts, event_times, device, (cudaStream_t)stream, false);
 }
 
 }  // extern "C"

@@ -18,8 +18,11 @@ attributes) under ../Results/<timestamp>/, but the time stepping runs on the B20
                      the device BDF kernel instead — LSODA leaves its Adams mode after ~25 steps on this stiff system
                      and is a variable-order BDF code from then on (csrc/bdf_batch.cu), `lband` / `uband` are then
                      ignored like `jac_sparsity`: the kernel's block-tridiagonal Jacobian is the exact structure;
-  other methods      (RK23, DOP853) SciPy-driven over the CUDA RHS — same arguments upstream passes (:104-109).
-                     MARLPDE_SCIPY_STEPPER=1 forces this route for every method.
+  method == "RK23"   the batched explicit Runge-Kutta kernel (csrc/erk_batch.cu), SciPy RK23 step for step: same
+  method == "DOP853" step control and error norm, the method's own dense output for t_eval and events (DOP853's
+                     three extra stages only in steps that need them, as SciPy);
+  MARLPDE_SCIPY_STEPPER=1 keeps SciPy's own stepper for every method, the RHS still evaluated by the CUDA kernel (one
+                     column per call) — same arguments upstream passes (:104-109).
 
 `integrate_equations_batch` is the sweep entry point: many parameter sets in one launch.
 """
@@ -65,22 +68,24 @@ def _build_model(pde_parms):
     return depths, eq, state.data.ravel()
 
 
-def _gpu_rk45(eq, y0, solver_parms, t_eval, n_cells):
-    """One column through the persistent kernel; returns an OdeResult look-alike."""
+def _gpu_rk45(eq, y0, solver_parms, t_eval, n_cells, integrate=None):
+    """One column through the persistent kernel (or `integrate`: the explicit RK23 / DOP853 kernel, same arguments and
+    result type); returns an OdeResult look-alike."""
     known = {"first_step", "atol", "rtol", "t_span", "method", "dense_output", "max_step"}
     extra = set(solver_parms) - known
     if extra:
-        raise TypeError(f"options not supported by the GPU RK45 path: {sorted(extra)}")
+        raise TypeError(f"options not supported by the GPU {solver_parms.get('method', 'RK45')} path: {sorted(extra)}")
+    integrate = integrate or _mb.integrate_rk45_batch
     # `dense_output=True` (parameters.py:221 has False) makes solve_ivp attach a callable OdeSolution as `sol.sol`;
     # upstream's driver never reads it (Evolve_scenario.py:104-183 uses sol.y, sol.t, sol.t_events only), so the flag is
     # accepted and stored with the other parameters; intermediate states come from `t_eval`, which IS the dense output
     # (quartic / cubic interpolant of the step, as SciPy) evaluated on the device.
     te = np.asarray(t_eval, dtype=np.float64) if t_eval is not None else np.array(solver_parms["t_span"], float)
-    res = _mb.integrate_rk45_batch(y0.reshape(1, 5, n_cells), eq.column_params, t_span=solver_parms["t_span"],
-                                   first_step=solver_parms.get("first_step", 1e-6),
-                                   rtol=solver_parms.get("rtol", 1e-3), atol=solver_parms.get("atol", 1e-6),
-                                   max_step=solver_parms.get("max_step", np.inf), t_eval=te,
-                                   events=True, event_capacity=4096)
+    res = integrate(y0.reshape(1, 5, n_cells), eq.column_params, t_span=solver_parms["t_span"],
+                    first_step=solver_parms.get("first_step", 1e-6),
+                    rtol=solver_parms.get("rtol", 1e-3), atol=solver_parms.get("atol", 1e-6),
+                    max_step=solver_parms.get("max_step", np.inf), t_eval=te,
+                    events=True, event_capacity=4096)
     k = int(res.next_eval[0])
     status = int(res.status[0])
     t_events = [np.sort(res.event_times[0, e, :min(int(res.event_counts[0, e]), res.event_times.shape[2])])
@@ -146,9 +151,10 @@ def integrate_equations(solver_parms, tracker_parms, pde_parms):
     start_computing = time.time()
     progress = 0
     scipy_stepper = os.environ.get("MARLPDE_SCIPY_STEPPER", "0") == "1"    # SciPy steps, the GPU only evaluates the RHS
-    if solver_parms["method"] == "RK45" and not scipy_stepper:
+    explicit = {"RK45": _mb.integrate_rk45_batch, "RK23": _mb.integrate_rk23_batch, "DOP853": _mb.integrate_dop853_batch}
+    if solver_parms["method"] in explicit and not scipy_stepper:
         gpu_parms = {k: v for k, v in solver_parms.items() if k not in ("jac_sparsity", "lband", "uband")}
-        sol = _gpu_rk45(eq, y0, gpu_parms, tracker_parms["t_eval"], n_cells)
+        sol = _gpu_rk45(eq, y0, gpu_parms, tracker_parms["t_eval"], n_cells, explicit[solver_parms["method"]])
         progress = (sol.t_reached - t0) / (end_time - t0)
     elif solver_parms["method"] == "Radau" and not scipy_stepper:
         sol = _gpu_implicit(eq, y0, solver_parms, tracker_parms["t_eval"], n_cells, "radau")
@@ -203,8 +209,8 @@ def integrate_equations(solver_parms, tracker_parms, pde_parms):
 def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_folder=None, device=0):
     """Parameter sweep: `pde_parms` is a Map_Scenario dictionary whose values may be arrays of
     shape (B,) (see marlpde_b200.sweep_lattice) or a list of such dictionaries.  All columns are
-    integrated in one launch of the kernel `method` selects (RK45: persistent on-chip kernel; Radau, BDF / LSODA: the
-    batched implicit kernels).  Returns the marlpde_b200.RK45Result / RadauResult;
+    integrated in one launch of the kernel `method` selects (RK45: persistent on-chip kernel; RK23, DOP853: the batched
+    explicit Runge-Kutta kernel; Radau, BDF / LSODA: the batched implicit kernels).  Returns the marlpde_b200.RK45Result / RadauResult;
     with `store_folder` one HDF5 file per sweep is written (datasets `solutions` (B,5,N,n_t),
     `times`, `status`, `nfev`, `n_accepted`, `n_rejected`, `next_eval`, `t_reached`, `event_counts`)."""
     if isinstance(pde_parms, (list, tuple)):
@@ -213,12 +219,13 @@ def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_fold
     solver_parms = dict(solver_parms)
     solver_parms.pop("backend", None)
     method = solver_parms.get("method", "RK45")
-    if method not in ("RK45", "Radau", "BDF", "LSODA"):
-        raise NotImplementedError("the batched on-device integrators implement method='RK45', 'Radau', 'BDF' and "
-                                  "'LSODA' (the latter on the BDF kernel: LSODA's stiff mode)")
+    if method not in ("RK45", "RK23", "DOP853", "Radau", "BDF", "LSODA"):
+        raise NotImplementedError("the batched on-device integrators implement method='RK45', 'RK23', 'DOP853', 'Radau', "
+                                  "'BDF' and 'LSODA' (the latter on the BDF kernel: LSODA's stiff mode)")
     params = _mb.derive_column_params(pde_parms)
     y0 = _mb.initial_state(pde_parms)
-    integrate = {"RK45": _mb.integrate_rk45_batch, "Radau": _mb.integrate_radau_batch}.get(method, _mb.integrate_bdf_batch)
+    integrate = {"RK45": _mb.integrate_rk45_batch, "RK23": _mb.integrate_rk23_batch, "DOP853": _mb.integrate_dop853_batch,
+                 "Radau": _mb.integrate_radau_batch}.get(method, _mb.integrate_bdf_batch)
     res = integrate(y0, params, t_span=solver_parms.get("t_span", (0, 1)),
                     first_step=solver_parms.get("first_step", 1e-6),
                     rtol=solver_parms.get("rtol", 1e-3), atol=solver_parms.get("atol", 1e-3),

@@ -13,4 +13,5 @@ The reference-facing drop-in (`Map_Scenario`, `Solver`, `Tracker`, `LMAHeureuxPo
 from . import _cabi  # noqa: F401
 from .params import derive_column_params, initial_state, sweep_lattice  # noqa: F401
 from .batch import rhs_batch, integrate_rk45_batch, integrate_radau_batch, integrate_bdf_batch, RK45Result, RadauResult  # noqa: F401
+from .batch import integrate_rk23_batch, integrate_dop853_batch  # noqa: F401
 from . import sweep  # noqa: F401

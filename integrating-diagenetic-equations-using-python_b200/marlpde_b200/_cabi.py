@@ -102,7 +102,21 @@ SYMBOLS = {
                                         _P, _P, _P, _P, _P, C.c_int]),
     "marlpde_bdf_integrate_async": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
                                               _P, _P, _P, _P, _P, C.c_int, _P]),
-    "marlpde_probe_jacobian": (C.c_int, [_P, _P, C.c_int, _P, C.c_int]),
+    "marlpde_rk23_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
+    "marlpde_rk23_integrate_dev": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                             _P, _P, _P, _P, _P, C.c_size_t, _P, _P]),
+    "marlpde_rk23_integrate": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                         _P, _P, _P, _P, C.c_int]),
+    "marlpde_rk23_integrate_async": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                               _P, _P, _P, _P, C.c_int, _P]),
+    "marlpde_dop853_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
+    "marlpde_dop853_integrate_dev": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                               _P, _P, _P, _P, _P, C.c_size_t, _P, _P]),
+    "marlpde_dop853_integrate": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                           _P, _P, _P, _P, C.c_int]),
+    "marlpde_dop853_integrate_async": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                                 _P, _P, _P, _P, C.c_int, _P]),
+    "marlpde_probe_jacobian":(C.c_int, [_P, _P, C.c_int, _P, C.c_int]),
     "marlpde_probe_math": (C.c_int, [C.c_int, _P, C.c_int, _P, C.c_int]),
     "marlpde_probe_fp64_peak": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double)]),
     "marlpde_rk45_integrate": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),

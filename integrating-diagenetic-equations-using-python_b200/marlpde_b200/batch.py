@@ -404,3 +404,101 @@ def _integrate_implicit(kind, y0, params, t_span, first_step, rtol, atol, t_eval
                        newton_iterations=stats[:, 2].copy(), newton_failures=stats[:, 3].copy(),
                        t_eval=t_eval_arr, snapshots=snaps, next_eval=st_out["next_eval"].copy(), event_counts=ec,
                        event_times=et, state=st_out)
+
+
+def integrate_rk23_batch(y0, params, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e-3, t_eval=None,
+                         max_step=np.inf, max_steps: int = 0, events: bool = False, event_capacity: int = 0,
+                         state: np.ndarray | None = None, device: int = 0, inplace: bool = False) -> RK45Result:
+    """Adaptive Bogacki-Shampine RK23 for every column (csrc/erk_batch.cu), SciPy `solve_ivp(method="RK23")` semantics
+    per column: same step-size control and error norm, cubic dense output for `t_eval` and event location.  Arguments
+    and result as for `integrate_rk45_batch` (no `quantum`); a column that stops on `max_steps` stops after an accepted
+    step and resumes from the returned `.state` and `.y` exactly as if it had not stopped."""
+    return _integrate_erk("rk23", y0, params, t_span, first_step, rtol, atol, t_eval, max_step, max_steps, events,
+                          event_capacity, state, device, inplace)
+
+
+def integrate_dop853_batch(y0, params, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e-3, t_eval=None,
+                           max_step=np.inf, max_steps: int = 0, events: bool = False, event_capacity: int = 0,
+                           state: np.ndarray | None = None, device: int = 0, inplace: bool = False) -> RK45Result:
+    """Adaptive Dormand-Prince DOP853 for every column (csrc/erk_batch.cu), SciPy `solve_ivp(method="DOP853")`
+    semantics per column, including the seventh-order dense output whose three extra RHS evaluations are spent (and
+    counted in `nfev`) only in steps that sample `t_eval` or locate an event.  Arguments and result as for
+    `integrate_rk23_batch`."""
+    return _integrate_erk("dop853", y0, params, t_span, first_step, rtol, atol, t_eval, max_step, max_steps, events,
+                          event_capacity, state, device, inplace)
+
+
+def _integrate_erk(kind, y0, params, t_span, first_step, rtol, atol, t_eval, max_step, max_steps, events,
+                   event_capacity, state, device, inplace) -> RK45Result:
+    lib = _cabi.lib()
+    f_ws = getattr(lib, f"marlpde_{kind}_workspace_bytes")
+    f_dev = getattr(lib, f"marlpde_{kind}_integrate_dev")
+    f_host = getattr(lib, f"marlpde_{kind}_integrate")
+    t0, t_bound = float(t_span[0]), float(t_span[1])
+    if not t_bound > t0:
+        raise ValueError("only forward integration (t_span[1] > t_span[0]) is supported")
+    if state is None:
+        fs = np.asarray(first_step, dtype=np.float64)
+        if np.any(fs <= 0):
+            raise ValueError("`first_step` must be positive.")
+        if np.any(fs > abs(t_bound - t0)):
+            raise ValueError("`first_step` exceeds bounds.")
+    t_eval_arr = np.zeros(0) if t_eval is None else np.ascontiguousarray(t_eval, dtype=np.float64)
+    if t_eval_arr.ndim != 1:
+        raise ValueError("`t_eval` must be 1-dimensional.")
+    if t_eval_arr.size:
+        if np.any(t_eval_arr < t0) or np.any(t_eval_arr > t_bound):
+            raise ValueError("Values in `t_eval` are not within `t_span`.")
+        if np.any(np.diff(t_eval_arr) <= 0):
+            raise ValueError("Values in `t_eval` are not properly sorted.")
+    n_eval = int(t_eval_arr.size)
+    cap = int(event_capacity) if events else 0
+    opts = _cabi.RK45Options(t_bound=t_bound, rtol=float(rtol), atol=float(atol), max_step=float(max_step),
+                             max_steps=int(max_steps), n_eval=n_eval, event_capacity=cap,
+                             flags=(_cabi.FLAG_EVENTS if events else 0) | _model_flags(params), quantum=0)
+    if _is_torch(y0):
+        import torch
+        if not y0.is_cuda or y0.dtype != torch.float64 or not y0.is_contiguous():
+            raise ValueError("device path needs a contiguous float64 CUDA tensor")
+        dev = y0.device
+        d_params = params if _is_torch(params) else params_to_device(params, dev)
+        B = d_params.numel() // PARAMS_DTYPE.itemsize
+        _check_y(y0, B)
+        N = y0.shape[2]
+        st = make_state(B, t0, first_step) if state is None else np.ascontiguousarray(state, dtype=STATE_DTYPE)
+        y = y0 if inplace else y0.clone()
+        with torch.cuda.device(dev):
+            d_state = torch.from_numpy(st.view(np.uint8).copy()).to(dev)
+            d_te = torch.from_numpy(t_eval_arr.copy()).to(dev) if n_eval else None
+            d_snap = torch.full((B, n_eval, 5, N), float("nan"), dtype=torch.float64, device=dev)   # rows >= next_eval stay NaN
+            d_queue = torch.zeros(1, dtype=torch.int32, device=dev)
+            d_ec = torch.zeros((B, NEVENTS), dtype=torch.int32, device=dev)
+            d_et = torch.full((B, NEVENTS, max(cap, 1)), float("nan"), dtype=torch.float64, device=dev)
+            nb = int(f_ws(B, N))
+            d_work = torch.empty(max(nb, 8) // 8, dtype=torch.float64, device=dev)
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.check(f_dev(
+                y.data_ptr(), d_params.data_ptr(), d_state.data_ptr(), B, N, C.byref(opts),
+                d_te.data_ptr() if n_eval else None, d_snap.data_ptr(), d_ec.data_ptr(), d_et.data_ptr(),
+                d_work.data_ptr(), nb, d_queue.data_ptr(), stream))
+            st_out = d_state.cpu().numpy().view(STATE_DTYPE).reshape(B)   # synchronises the stream
+            ec, et = d_ec.cpu().numpy(), d_et.cpu().numpy()[:, :, :cap]
+        snaps = d_snap
+    else:
+        p = _as_params(params)
+        B = p.shape[0]
+        y = np.array(y0, dtype=np.float64, order="C", copy=not inplace)
+        _check_y(y, B)
+        N = y.shape[2]
+        st_out = make_state(B, t0, first_step) if state is None else np.array(state, dtype=STATE_DTYPE, copy=True)
+        snaps = np.full((B, n_eval, 5, N), np.nan)
+        ec = np.zeros((B, NEVENTS), dtype=np.int32)
+        et = np.full((B, NEVENTS, cap), np.nan)
+        _cabi.check(f_host(
+            _cabi.ptr(y), _cabi.ptr(p), _cabi.ptr(st_out), B, N, C.byref(opts),
+            _cabi.ptr(t_eval_arr) if n_eval else None, _cabi.ptr(snaps) if n_eval else None,
+            _cabi.ptr(ec), _cabi.ptr(et) if cap else None, device))
+    return RK45Result(y=y, t=st_out["t"].copy(), h_abs=st_out["h_abs"].copy(), status=st_out["status"].copy(),
+                      n_accepted=st_out["n_accepted"].copy(), n_rejected=st_out["n_rejected"].copy(),
+                      nfev=st_out["nfev"].copy(), t_eval=t_eval_arr, snapshots=snaps,
+                      next_eval=st_out["next_eval"].copy(), event_counts=ec, event_times=et, state=st_out)

@@ -39,7 +39,10 @@ def predicted_cost(pde: dict, method: str = "RK45") -> np.ndarray:
     Radau: the implicit integrator does not see that limit; its work (step attempts incl. failed Newton episodes) is
     governed by how sharp the porosity front gets, i.e. by the compaction coefficient b (dPhi ~ 1/b).  Empirical fit on
     the 4096-column benchmark lattice (default base, r02o): work ~ b^2.16 S^-0.66 DCO3^0.05, rank correlation 0.996 —
-    the a-priori RK45 estimate has correlation 0.13 with it."""
+    the a-priori RK45 estimate has correlation 0.13 with it.
+    RK23, DOP853: the explicit estimate of RK45 — every explicit method is held at its stability limit on this system —
+    NOT fitted for these methods (their stability regions differ from RK45's only by a constant factor, which does not
+    change the order)."""
     if method in ("Radau", "BDF"):    # (BDF: same front-sharpness dependence; not fitted separately)
         b = np.atleast_1d(np.asarray(pde["b"], dtype=np.float64))
         srate = np.atleast_1d(np.asarray(pde["sedimentationrate"], dtype=np.float64))
@@ -132,8 +135,8 @@ def sweep_bdf(pde: dict, **kw) -> SweepResult:
 def sweep_rk45(pde: dict, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e-3, t_eval=None,
                events: bool = True, balance: bool = True, group=None, device=None, integrate=None,
                method: str = "RK45", **kw) -> SweepResult:
-    """Integrate every column of the sweep dictionary `pde` with the on-device RK45 (or, method="Radau", the implicit
-    integrator), sharded over the ranks of `group` (all ranks call this with the same arguments).  `integrate` is the
+    """Integrate every column of the sweep dictionary `pde` with the on-device RK45 (or the integrator `method` names:
+    "RK23", "DOP853", "Radau", "BDF"), sharded over the ranks of `group` (all ranks call this with the same arguments).  `integrate` is the
     per-rank batched integrator (default: marlpde_b200.integrate_{rk45,radau}_batch on `device`)."""
     import torch
     import torch.distributed as dist
@@ -152,10 +155,12 @@ def sweep_rk45(pde: dict, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e
     local = shard(pde, mine) if B > 1 else pde
 
     if integrate is None:
-        from .batch import integrate_bdf_batch, integrate_radau_batch, integrate_rk45_batch
-        if method not in ("RK45", "Radau", "BDF"):
-            raise ValueError("method must be 'RK45', 'Radau' or 'BDF'")
-        run = {"RK45": integrate_rk45_batch, "Radau": integrate_radau_batch, "BDF": integrate_bdf_batch}[method]
+        from .batch import (integrate_bdf_batch, integrate_dop853_batch, integrate_radau_batch, integrate_rk23_batch,
+                            integrate_rk45_batch)
+        run = {"RK45": integrate_rk45_batch, "RK23": integrate_rk23_batch, "DOP853": integrate_dop853_batch,
+               "Radau": integrate_radau_batch, "BDF": integrate_bdf_batch}.get(method)
+        if run is None:
+            raise ValueError("method must be 'RK45', 'RK23', 'DOP853', 'Radau' or 'BDF'")
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
 
         def integrate(y0, P, **opts):
