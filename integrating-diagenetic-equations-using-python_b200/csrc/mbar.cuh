@@ -4,7 +4,6 @@
 // neighbours, and only then waits — the barrier latency hides behind useful fp64 work.
 #pragma once
 #include <cstdint>
-#include <cstring>
 
 // the kernel's dynamic shared memory (the host emulator of tests/emu/ substitutes its own buffer)
 #ifndef MARLPDE_DYN_SMEM
@@ -25,13 +24,6 @@ namespace marlpde {
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) { ::simt::mbar_init(bar, count); }
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) { ::simt::mbar_arrive(bar); }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) { ::simt::mbar_wait(bar, parity); }
-// bulk copies complete at once on the host: expect_tx is then just the issuing thread's arrival
-__device__ __forceinline__ void mbar_fence_init() {}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, unsigned) { ::simt::mbar_arrive(bar); }
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t*) { std::memcpy(dst, src, bytes); }
-__device__ __forceinline__ void bulk_s2g(void* dst, const void* src, unsigned bytes) { std::memcpy(dst, src, bytes); }
-__device__ __forceinline__ void bulk_commit_wait() {}
-__device__ __forceinline__ void fence_proxy_async() {}
 #else
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
@@ -54,28 +46,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
         : "memory");
   } while (!done);
 }
-// ---- 1-D bulk copies of the TMA unit (cp.async.bulk, SASS UBLKCP): addresses and sizes are multiples of 16 bytes --------
-// makes a fresh mbarrier.init visible to the async proxy before a bulk copy signals the barrier
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-// one arrival + the number of bytes the bulk copies will deliver: the phase completes when both are in
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* dst, const void* src, unsigned bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit_wait() {      // all bulk stores of this thread have been written
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-  asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-// generic-proxy shared-memory writes become visible to the async proxy (before a bulk store reads them)
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 #endif
 
 }  // namespace marlpde

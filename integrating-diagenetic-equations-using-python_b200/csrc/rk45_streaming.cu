@@ -3,27 +3,24 @@
 //
 // Same stepper as rk45_persistent.cu (scipy RK45 semantics per column: rk.py `_step_impl`, `rk_step`,
 // `RkDenseOutput`; call site marlpde/Evolve_scenario.py:104-109) and the same rhs_pair arithmetic, but
-// the stage vectors stream through HBM/L2 instead of living on chip:
-//   * state, stage derivatives K1..K7 and two alternating stage-input vectors are [column][field][cell]
-//     arrays in a caller-provided workspace; a thread owns two adjacent cells, a CTA 256 cells of one
-//     column, the grid covers every column: 1.28 M cells in flight for 64 columns of 20 000 cells;
-//   * one launch per Runge-Kutta stage.  A stage kernel reads its input vector (own cells as 16-byte
-//     loads, the two halo cells from the neighbours' cache lines), evaluates the RHS, writes K_s and
-//     the next stage's input for its own cells.  The kernel boundary is the only synchronisation a
-//     stage needs (halos), so columns never wait for each other inside a kernel;
-//   * per-column control (error norm from per-CTA partial sums added in fixed order, accept/reject,
+// a column is cut into overlapping windows and only y and the stage derivatives stream through HBM/L2:
+//   * state, stage derivatives K1..K7 and a second y buffer are [column][field][cell] arrays in a
+//     caller-provided workspace; an accepted step writes y_new to the y buffer not in use and flips
+//     the index instead of copying;
+//   * ONE launch of tile_attempt_kernel per step attempt: a CTA integrates one window of a column
+//     through all six stages and the FSAL evaluation on chip (see below) and writes y_new, K7 and its
+//     window's contribution to the error norm.  The kernel boundary is the only synchronisation
+//     between windows, so columns never wait for each other inside a kernel;
+//   * per-column control (error norm from per-window partial sums added in fixed order, accept/reject,
 //     step-size factor, t_eval dense output, FSAL by swapping two slot indices instead of copying K7)
-//     is folded into the `prepare` kernel that also forms the stage-2 input of the next attempt.
-//     Control blocks are double buffered, so every CTA of a column derives the same decision from
-//     the same inputs while the column's first CTA publishes the updated block;
-//   * algorithmic HBM traffic: 42 vector passes of 40 bytes per cell and attempt = 1 680 B per cell
+//     runs in the prologue of the next attempt's launch (close_and_begin); prepare_kernel closes the
+//     last attempt of a call.  Control blocks are double buffered, so every CTA of a column derives
+//     the same decision from the same inputs while the column's first CTA publishes the updated block;
+//   * algorithmic HBM traffic: 4 vector passes of 40 bytes per cell and attempt = 160 B per cell
 //     (DESIGN.md §4.4); the L2 keeps working sets up to ~100 MB on chip.
 // A call enqueues a fixed number of step attempts (no host round trip, no synchronisation); columns
 // that reach t_bound earlier idle, columns that do not come back resumable with status STEP_BUDGET.
-//
-// Default since r01c: the six stage launches of an attempt are replaced by ONE launch of
-// tile_attempt_kernel (overlapped 640-cell windows integrated on chip, see below); the per-stage
-// kernels remain as the HBM-streaming variant (MARLPDE_RK45_STREAM=stages) and for K1 = f(y).
+// K1 = f(y) of the first attempt comes from k1_kernel.
 #include <cuda_runtime.h>
 
 #include <cstdint>
@@ -54,11 +51,11 @@ struct Ctl {                                   // per-column control block (doub
   int k1, k7;                                  // physical slots of K1 and K7 (0 or 6)
   int fresh;                                   // 1: K1 has just been evaluated, no attempt finished yet
   int midstep;                                 // resumed inside a step (after a rejected attempt)
-  int ysl;                                     // tile path: which buffer holds y (0: caller's y, 1: workspace vector 0)
+  int ysl;                                     // which buffer holds y (0: caller's y, 1: workspace vector 0)
   int locate;                                  // events: 1 = the accepted step in flight has a sign change; the attempt
                                                // is replayed with K3..K6 stored, then its roots are located and it commits
   unsigned ev_prev;                            // predicate bits of the monitors at the start of the current step
-  int skip;                                    // tile path: the attempt described here has NOT been run yet (the launch that
+  int skip;                                    // the attempt described here has NOT been run yet (the launch that
                                                // located the events of the previous step ran no attempt): nothing to close
 };
 
@@ -69,22 +66,24 @@ struct Args {
   const double* t_eval;
   double* snap;
   double* K;                 // [7][B][5][N]
-  double* tile;              // [2][B][5][N]
+  double* tile;              // [B][5][N] second y buffer (workspace vector 0)
   double* partials;          // [2][B][pstride]: written by the launch that runs an attempt under control buffer p into
-                             // parity p, read by the launch that closes it (the fused tile kernel closes the previous
+                             // parity p, read by the launch that closes it (the tile kernel closes the previous
                              // attempt in its prologue while faster CTAs of the same launch already write the next sums)
   Ctl* ctl;                  // [2][B]
   unsigned* evpart;          // [2][B][pstride] predicate bits of the monitors per CTA / window (MARLPDE_FLAG_EVENTS)
   int32_t* ev_counts;        // [B][7]
   double* ev_times;          // [B][7][event_capacity]
   int B, N, tiles;
-  int tiles2;                // overlapped-tile path: attempt tiles per column (0: one launch per stage)
+  int tiles2;                // tile_attempt_kernel windows per column
   int pstride;               // entries per column in `partials` and `evpart`
   marlpde_rk45_options opt;
 };
 
 __host__ __device__ inline size_t align256(size_t x) { return (x + 255) / 256 * 256; }
 
+// Workspace layout (marlpde_rk45_stream_workspace_bytes).  Of the two vectors at off_tile only the first is used (the
+// second y buffer); the second slot is kept so that the workspace size seen through the C ABI does not change.
 struct Layout {
   size_t off_K, off_tile, off_part, off_ctl, off_ev, total;
 };
@@ -189,8 +188,8 @@ __device__ __forceinline__ Cells my_cells(const Args& A) {
   return m;
 }
 
-// tile path: y ping-pongs between the caller's array and workspace vector 0 (an accepted step flips the index
-// instead of copying y_new over y); the per-stage path keeps y in the caller's array
+// y ping-pongs between the caller's array and workspace vector 0 (an accepted step flips the index instead of copying
+// y_new over y)
 __device__ __forceinline__ double* ybuf(const Args& A, int sl) { return sl ? A.tile : A.y; }
 
 // two adjacent cells of field f from a [B][5][N] vector (N may be odd: no 16-byte loads)
@@ -205,7 +204,7 @@ __device__ __forceinline__ void st2(double* v, const Cells& m, int f, int N, dou
   if (m.v1) p[1] = b;
 }
 
-// tile path, end of a call: columns whose y lives in the workspace buffer are copied back to the caller's array
+// end of a call: columns whose y lives in the workspace buffer are copied back to the caller's array
 __global__ void __launch_bounds__(kThreads) copyback_kernel(const Args A, int parity) {
   const Cells m = my_cells(A);
   if (A.ctl[(size_t)parity * A.B + m.col].ysl == 0) return;
@@ -315,9 +314,9 @@ __device__ void locate_events(const Args& A, const Ctl& c, int col, unsigned act
 // publishes the new control block in `pin ^ 1` (first CTA of the column) and returns it: every CTA of a column derives
 // the same block from the same inputs.  `m` = the cells this THREAD writes dense-output samples for.  Called by every
 // thread of the CTA (the event location inside has block barriers).  `run` = whether the attempt described by the
-// returned block is to be run by the caller now (tile path only; false for a column that is done, and for the launch
-// in which the events of a step were located: the locating CTA reads every cell's stage derivatives, so no CTA of the
-// column may start overwriting them).
+// returned block is to be run by the caller now (false for a column that is done, and for the launch in which the
+// events of a step were located: the locating CTA reads every cell's stage derivatives, so no CTA of the column may
+// start overwriting them).
 __device__ Ctl close_and_begin(const Args& A, int pin, const Cells& m, bool first_cta, const fm::Tables& tb, bool& run) {
   const int N = A.N;
   const size_t vec = (size_t)A.B * 5 * N;
@@ -336,13 +335,11 @@ __device__ Ctl close_and_begin(const Args& A, int pin, const Cells& m, bool firs
     return c;
   }
   bool located = false;
-  double* const tile0 = A.tile;
-  double* const tile1 = A.tile + vec;
-  const double* K1 = A.K + (size_t)c.k1 * vec;
+  const double* const K1 = A.K + (size_t)c.k1 * vec;
   if (!c.fresh) {
-    // ---- error norm of the attempt that just ran: per-CTA partial sums, fixed order
+    // ---- error norm of the attempt that just ran: per-window partial sums, fixed order
     double sum = 0.0;
-    const int n_part = A.tiles2 > 0 ? A.tiles2 : A.tiles;
+    const int n_part = A.tiles2;
     const double* part = partials_of(A, pin, m.col);
     for (int i = 0; i < n_part; ++i) sum += part[i];
     const double err_norm = sqrt(sum / (double)(5 * N));
@@ -419,22 +416,11 @@ __device__ Ctl close_and_begin(const Args& A, int pin, const Cells& m, bool firs
         ++ne;
       }
       c.next_eval = ne;
-      // accept: y <- y_new, K1 <-> K7.  Tile path: y_new was written to the other y buffer, flip the index;
-      // per-stage path: y_new is the stage-6 input (tile 0), copy it over y
-      if (A.tiles2 > 0) {
-        c.ysl ^= 1;
-      } else {
-#pragma unroll
-        for (int f = 0; f < 5; ++f) {
-          double a, b;
-          ld2(tile0, m, f, N, a, b);
-          st2(A.y, m, f, N, a, b);
-        }
-      }
+      // accept: y <- y_new (written to the other y buffer: flip the index), K1 <-> K7
+      c.ysl ^= 1;
       const int tmp = c.k1;
       c.k1 = c.k7;
       c.k7 = tmp;
-      K1 = A.K + (size_t)c.k1 * vec;
       c.t = c.t_new;
       c.h_abs *= factor;
       c.n_acc += 1;
@@ -473,25 +459,14 @@ __device__ Ctl close_and_begin(const Args& A, int pin, const Cells& m, bool firs
       c.status = MARLPDE_STATUS_STEP_TOO_SMALL;
     }
   }
-  if (c.active && A.tiles2 == 0) {
-    // stage-2 input: y + h a21 K1 (for an accepted step y was just rewritten by this very thread)
-    const double ha = c.h * dp::a21;
-#pragma unroll
-    for (int f = 0; f < 5; ++f) {
-      double y0, y1, k0, k1v;
-      ld2(A.y, m, f, N, y0, y1);
-      ld2(K1, m, f, N, k0, k1v);
-      st2(tile1, m, f, N, fma(ha, k0, y0), fma(ha, k1v, y1));
-    }
-  }
   run = c.active != 0 && !located;
-  if (A.tiles2 > 0 && c.active && located) c.skip = 1;      // the attempt begun here runs in the NEXT launch
+  if (c.active && located) c.skip = 1;                      // the attempt begun here runs in the NEXT launch
   if (publisher) A.ctl[(size_t)(pin ^ 1) * A.B + m.col] = c;
   return c;
 }
 
-// ---- prepare: close_and_begin as a kernel of its own — the one-launch-per-stage variant runs it before every attempt,
-// the tile path (whose attempt kernel does this in its prologue) only once, to close the last attempt of a batch.
+// ---- prepare: close_and_begin as a kernel of its own, to close the last attempt of a batch (the attempt kernel closes
+// every earlier one in its prologue).
 __global__ void __launch_bounds__(kThreads) prepare_kernel(const Args A, int pin) {
   __shared__ __align__(16) unsigned char tab_raw[fm::kTableBytes];
   const fm::Tables tb = fm::stage_tables(tab_raw, threadIdx.x, blockDim.x);
@@ -501,83 +476,27 @@ __global__ void __launch_bounds__(kThreads) prepare_kernel(const Args A, int pin
   close_and_begin(A, pin, m, blockIdx.x == m.col * A.tiles, tb, run);
 }
 
-// Stage algebra as data: after K_{i+1} = r has been evaluated, the next stage input is
-//   y + h (sum_j kCoef[i][j-1] K_j + kNew[i] r)          (i = 1..5; i = 5 gives y_new)
-// and for i = 6 the same sum is the error estimate h (sum_j e_j K_j + e_7 r).
-__constant__ double kCoef[7][6] = {{0, 0, 0, 0, 0, 0},
-                                   {dp::a31, 0, 0, 0, 0, 0},
-                                   {dp::a41, dp::a42, 0, 0, 0, 0},
-                                   {dp::a51, dp::a52, dp::a53, 0, 0, 0},
-                                   {dp::a61, dp::a62, dp::a63, dp::a64, 0, 0},
-                                   {dp::b1, 0, dp::b3, dp::b4, dp::b5, 0},
-                                   {dp::e1, 0, dp::e3, dp::e4, dp::e5, dp::e6}};
-__constant__ double kNew[7] = {0, dp::a32, dp::a43, dp::a54, dp::a65, dp::b6, dp::e7};
-
-// ---- one Runge-Kutta stage: i = 0 evaluates K1 = f(y) (fresh columns), i = 1..6 evaluates K_{i+1}
-// from stage-input vector (i & 1), stores it and writes the next stage input; i = 6 writes the
-// CTA's contribution to the error norm instead.
-// Memory-level parallelism: EVERYTHING the stage reads — its input cells and halos, y and the
-// earlier K's — is requested before the RHS is evaluated (the K's are reduced to one partial sum
-// per cell on arrival), so ~80 independent loads per thread are in flight while the fp64 work of
-// the RHS runs; after the RHS only two fused multiply-adds and the stores remain.
-__global__ void __launch_bounds__(kThreads, 3) stage_kernel(const Args A, int i, int cbuf) {
+// ---- K1 = f(y) at the start of a call (columns still active), and the monitor bits at the start point.  256 cells per
+// CTA; a thread's own cells and the two halo cells are read from y in HBM.
+__global__ void __launch_bounds__(kThreads, 3) k1_kernel(const Args A) {
   __shared__ ColumnConsts kc;
   __shared__ __align__(16) unsigned char tab_raw[fm::kTableBytes];
-  __shared__ double red[kThreads / 32];
   const Cells m = my_cells(A);
-  const Ctl c = A.ctl[(size_t)cbuf * A.B + m.col];
-  if (!c.active || (i == 0 && !c.fresh)) return;          // uniform per CTA
+  const Ctl c = A.ctl[m.col];                               // control buffer 0, as init_kernel left it
+  if (!c.active || !c.fresh) return;                        // uniform per CTA
   const fm::Tables tb = fm::stage_tables(tab_raw, threadIdx.x, blockDim.x);
   const int N = A.N;
   if (threadIdx.x == 0) make_consts(A.params[m.col], N, kc);
   const size_t vec = (size_t)A.B * 5 * N;
-  const double* in = i == 0 ? A.y : A.tile + (size_t)(i & 1) * vec;
-  double* const nxt = A.tile + (size_t)((i + 1) & 1) * vec;
-  const double h = c.h;
-  auto Kslot = [&](int logical) -> double* {   // logical stage 1..7 -> physical slot
-    const int s = logical == 1 ? c.k1 : (logical == 7 ? c.k7 : logical - 1);
-    return A.K + (size_t)s * vec;
-  };
 
-  // ---- all loads of this stage: input cells + raw halo values, y, earlier K's (as partial sums)
-  double cc[5][2], hm[5], hp[5], acc[5][2], pre[5][2];
+  double cc[5][2], hm[5], hp[5];
 #pragma unroll
   for (int f = 0; f < 5; ++f) {
-    const double* p = in + m.base + (size_t)f * N;
+    const double* p = A.y + m.base + (size_t)f * N;
     cc[f][0] = m.v0 ? p[0] : 0.5;
     cc[f][1] = m.v1 ? p[1] : 0.5;
     hm[f] = (m.v0 && m.cell0 > 0) ? p[-1] : 0.0;
     hp[f] = (m.cell0 + 2 < N) ? p[2] : 0.0;
-    acc[f][0] = acc[f][1] = 0.0;
-    pre[f][0] = pre[f][1] = 0.0;
-  }
-  if (i > 0) {
-#pragma unroll
-    for (int j = 1; j <= 6; ++j) {
-      const double cj = kCoef[i][j - 1];
-      if (cj != 0.0) {                                      // uniform: the stage index is a launch argument
-        const double* Kj = Kslot(j);
-#pragma unroll
-        for (int f = 0; f < 5; ++f) {
-          double a0, a1;
-          ld2(Kj, m, f, N, a0, a1);
-          acc[f][0] = fma(cj, a0, acc[f][0]);
-          acc[f][1] = fma(cj, a1, acc[f][1]);
-        }
-      }
-    }
-#pragma unroll
-    for (int f = 0; f < 5; ++f) {
-      double y0, y1;
-      ld2(A.y, m, f, N, y0, y1);
-      if (i < 6) {
-        pre[f][0] = fma(h, acc[f][0], y0);
-        pre[f][1] = fma(h, acc[f][1], y1);
-      } else {   // error weights h / scale, scale = atol + rtol max(|y|, |y_new|)  (cc = y_new)
-        pre[f][0] = h * fm::rcp3(fma(fmax(fabs(y0), fabs(cc[f][0])), A.opt.rtol, A.opt.atol));
-        pre[f][1] = h * fm::rcp3(fma(fmax(fabs(y1), fabs(cc[f][1])), A.opt.rtol, A.opt.atol));
-      }
-    }
   }
   __syncthreads();                                          // kc and the tables are staged
 
@@ -597,56 +516,24 @@ __global__ void __launch_bounds__(kThreads, 3) stage_kernel(const Args A, int i,
   const bool in_mask[2] = {m.cell0 >= kc.mask_lo && m.cell0 < kc.mask_hi,
                            m.cell0 + 1 >= kc.mask_lo && m.cell0 + 1 < kc.mask_hi};
   double r[5][2], U[2], W[2];
-  // (kVarDPhi = true: bit-identical for columns without MARLPDE_MODEL_VAR_DPHI; this kernel is bound by HBM traffic)
+  // (kVarDPhi = true: bit-identical for columns without MARLPDE_MODEL_VAR_DPHI; runs once per call)
   PairFlags fl = rhs_pair<rhs_schedule(kSchedSplit), true>(kc, tb, cc, mlo, phi, in_mask, r, U, W);
   fl.bad[0] = fl.bad[0] && m.v0;
   fl.bad[1] = fl.bad[1] && m.v1;
   if (fl.bad[0] || fl.bad[1]) rhs_pair_fixup(kc, tb, fl, cc, mlo, phi, in_mask, r, U, W);
 
-  // ---- epilogue: K_{i+1} and the next stage input (or the error contribution)
-  double part = 0.0;
-  if (i == 0) {
-    double* K1 = Kslot(1);
+  double* const K1 = A.K + (size_t)c.k1 * vec;
 #pragma unroll
-    for (int f = 0; f < 5; ++f) st2(K1, m, f, N, r[f][0], r[f][1]);
-    if (A.opt.flags & MARLPDE_FLAG_EVENTS) {               // monitor signs at the start point (U, W come with K1)
-      __shared__ unsigned sbits[kThreads / 32];
-      const unsigned bw = __reduce_or_sync(0xffffffffu, event_bits_sel(cc, U, W, m.v0, m.v1));
-      if ((threadIdx.x & 31) == 0) sbits[threadIdx.x >> 5] = bw;
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        unsigned b = 0u;
-        for (int w = 0; w < kThreads / 32; ++w) b |= sbits[w];
-        evpart_of(A, cbuf, m.col)[blockIdx.x - m.col * A.tiles] = b;
-      }
-    }
-  } else if (i < 6) {
-    double* Kn = Kslot(i + 1);
-    const double hn = h * kNew[i];
-#pragma unroll
-    for (int f = 0; f < 5; ++f) {
-      st2(Kn, m, f, N, r[f][0], r[f][1]);
-      st2(nxt, m, f, N, fma(hn, r[f][0], pre[f][0]), fma(hn, r[f][1], pre[f][1]));
-    }
-  } else {
-    double* K7 = Kslot(7);
-#pragma unroll
-    for (int f = 0; f < 5; ++f) {
-      st2(K7, m, f, N, r[f][0], r[f][1]);
-      const double z0 = fma(kNew[6], r[f][0], acc[f][0]) * pre[f][0];
-      const double z1 = fma(kNew[6], r[f][1], acc[f][1]) * pre[f][1];
-      if (m.v0) part = fma(z0, z0, part);
-      if (m.v1) part = fma(z1, z1, part);
-    }
-    // CTA-wide sum in a fixed order: xor butterfly per warp, then the warp sums in warp order
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = part;
+  for (int f = 0; f < 5; ++f) st2(K1, m, f, N, r[f][0], r[f][1]);
+  if (A.opt.flags & MARLPDE_FLAG_EVENTS) {                 // monitor signs at the start point (U, W come with K1)
+    __shared__ unsigned sbits[kThreads / 32];
+    const unsigned bw = __reduce_or_sync(0xffffffffu, event_bits_sel(cc, U, W, m.v0, m.v1));
+    if ((threadIdx.x & 31) == 0) sbits[threadIdx.x >> 5] = bw;
     __syncthreads();
     if (threadIdx.x == 0) {
-      double s = 0.0;
-      for (int w = 0; w < kThreads / 32; ++w) s += red[w];
-      partials_of(A, cbuf, m.col)[blockIdx.x - m.col * A.tiles] = s;
+      unsigned b = 0u;
+      for (int w = 0; w < kThreads / 32; ++w) b |= sbits[w];
+      evpart_of(A, 0, m.col)[blockIdx.x - m.col * A.tiles] = b;
     }
   }
 }
@@ -658,8 +545,8 @@ __global__ void __launch_bounds__(kThreads, 3) stage_kernel(const Args A, int i,
 // persistent kernel (y, K1, stage input and stage derivative in registers, K2..K5 and the halo
 // exchange tile in shared memory).  Neighbouring windows overlap by 2 x 6 cells: a stage evaluation
 // invalidates one more cell at each window edge (its neighbour lies outside the window), so after
-// K2..K7 the inner 628 cells are exact and only those are written back.  HBM traffic per attempt drops
-// from 42 to 4 vector passes (read y, K1; write y_new, K7), at 1.9 % redundant arithmetic.
+// K2..K7 the inner 628 cells are exact and only those are written back.  HBM traffic per attempt is
+// 4 vector passes (read y, K1; write y_new, K7), at 1.9 % redundant arithmetic.
 // =================================================================================================
 // Window sizes: 320 threads (640-cell windows, 628 owned cells) when the batch fills the machine; 128 threads (256-cell
 // windows, 244 owned) for small batches — N = 20 000 x 1 is 32 large windows on 148 SMs, and an attempt cannot be
@@ -669,11 +556,7 @@ constexpr int kTileHalo = 6;
 constexpr int kTileThreadsLarge = 320, kTileThreadsSmall = 128;
 __host__ __device__ constexpr int tile_valid_cells(int threads) { return 2 * threads - 2 * kTileHalo; }
 
-// TMA: the window loads / write-back go through the TMA unit (1-D bulk copies, UBLKCP) and a shared-memory staging
-// area instead of per-thread loads and stores.  Measured on B200 (r02a): 208 k against 231 k column-steps/s at
-// N = 20 000 x 64 — the kernel is bound by the fp64 pipe and its DRAM traffic already equals the algorithmic traffic, so
-// the staging hop only adds shared-memory traffic.  Shipped and selectable (MARLPDE_RK45_TILE_TMA=1), off by default.
-template <int TT, bool TMA>
+template <int TT>
 struct TileSmemT {
   static constexpr size_t off_K = 0;                                                   // double2 [4][5][TT]
   static constexpr size_t off_E = off_K + sizeof(double2) * 4 * 5 * TT;                // double [2][5][TT]
@@ -681,17 +564,16 @@ struct TileSmemT {
   static constexpr size_t off_tab = off_O + sizeof(double) * 2 * 5 * TT;
   static constexpr size_t off_kc = off_tab + fm::kTableBytes;
   static constexpr size_t off_red = off_kc + (sizeof(ColumnConsts) + 15) / 16 * 16;
-  static constexpr size_t off_bar = off_red + 16 * sizeof(double);                      // two mbarriers
-  static constexpr size_t off_stage = off_bar + 16;                                    // double [2][5][2 TT] (TMA)
-  static constexpr size_t total = off_stage + (TMA ? sizeof(double) * 2 * 5 * 2 * TT : 0);
-  static_assert(off_stage % 16 == 0 && total <= 227 * 1024, "tile kernel shared memory");
+  static constexpr size_t off_bar = off_red + 16 * sizeof(double);                      // mbarrier
+  static constexpr size_t total = off_bar + 16;
+  static_assert(total <= 227 * 1024, "tile kernel shared memory");
 };
 
 // VD: batches with MARLPDE_MODEL_VAR_DPHI columns (opt.flags & MARLPDE_FLAG_VAR_DPHI); EV: MARLPDE_FLAG_EVENTS
-template <bool VD, bool EV, int TT, bool TMA>
+template <bool VD, bool EV, int TT>
 __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int pin) {
   MARLPDE_DYN_SMEM(smem_raw);
-  using TileSmem = TileSmemT<TT, TMA>;
+  using TileSmem = TileSmemT<TT>;
   constexpr int kTileThreads = TT, kTileCells = 2 * TT, kTileValid = tile_valid_cells(TT);
   constexpr int TP = kTileThreads;
   const int tid = threadIdx.x;
@@ -729,28 +611,6 @@ __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int p
   if (tid == 0) make_consts(A.params[col], N, kc);
   const size_t vec = (size_t)A.B * 5 * N;
   const double h = c0.h;
-  // Window loads and write-back by the TMA unit: ten 1-D bulk copies each way (5 fields x {y, K1} in, {y_new, K7} out) issued
-  // by one thread, in flight while the tables and the column constants are set up.  Every row start and length is a
-  // multiple of 16 bytes when N is even (window starts and the 628-cell stride are even); odd N keeps the plain loads.
-  double* const sStage = reinterpret_cast<double*>(smem_raw + TileSmem::off_stage);
-  uint64_t* const sLoad = sBar + 1;
-  const bool tma = TMA && (N & 1) == 0 && ((reinterpret_cast<uintptr_t>(A.y) | reinterpret_cast<uintptr_t>(A.K) |
-                                             reinterpret_cast<uintptr_t>(A.tile)) & 15) == 0;   // (a caller's view may be 8-byte aligned)
-  const int w0 = tile * kTileValid - kTileHalo;              // global cell of window position 0
-  if (TMA && tma && tid == 0) {
-    const int lo = w0 < 0 ? 0 : w0, hi = w0 + kTileCells < N ? w0 + kTileCells : N;
-    const unsigned bytes = (unsigned)(hi - lo) * 8u;
-    mbar_init(sLoad, 1);
-    mbar_fence_init();
-    mbar_arrive_expect_tx(sLoad, 10u * bytes);
-    const size_t row0 = (size_t)col * 5 * N + (size_t)lo;
-    const double* const ysrc = ybuf(A, c0.ysl) + row0;
-    const double* const ksrc = A.K + (size_t)c0.k1 * vec + row0;
-    for (int f = 0; f < 5; ++f) {
-      bulk_g2s(sStage + f * kTileCells + (lo - w0), ysrc + (size_t)f * N, bytes, sLoad);
-      bulk_g2s(sStage + (5 + f) * kTileCells + (lo - w0), ksrc + (size_t)f * N, bytes, sLoad);
-    }
-  }
 
   const int e0 = 2 * tid;                                   // position inside the window
   const int g0 = tile * kTileValid - kTileHalo + e0;        // global cell of my first cell (always even)
@@ -773,19 +633,7 @@ __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int p
   auto Kld = [&](int s, int f) -> double2 { return sK[(s * 5 + f) * TP]; };
 
   double y[5][2], k1[5][2], c[5][2], r[5][2];
-  if (TMA && tma) {
-    __syncthreads();                                        // the load barrier is initialised
-    mbar_wait(sLoad, 0);                                    // ... and the ten rows have landed
-#pragma unroll
-    for (int f = 0; f < 5; ++f) {                           // (positions outside the column hold stale bytes: not selected)
-      const double2 yv = *reinterpret_cast<const double2*>(sStage + f * kTileCells + e0);
-      const double2 kv = *reinterpret_cast<const double2*>(sStage + (5 + f) * kTileCells + e0);
-      y[f][0] = in0 ? yv.x : 0.5;
-      y[f][1] = in1 ? yv.y : 0.5;
-      k1[f][0] = in0 ? kv.x : 0.0;
-      k1[f][1] = in1 ? kv.y : 0.0;
-    }
-  } else {
+  {
     const double* K1g = Kslot(1);
 #pragma unroll
     for (int f = 0; f < 5; ++f) {
@@ -929,18 +777,13 @@ __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int p
     if (out0) part = fma(z0, z0, part);
     if (out1) part = fma(z1, z1, part);
     const size_t o = base + (size_t)f * N;
-    if (TMA && tma) {                                        // staged; one thread stores the owned range below
-      *reinterpret_cast<double2*>(sStage + f * kTileCells + e0) = make_double2(c[f][0], c[f][1]);
-      *reinterpret_cast<double2*>(sStage + (5 + f) * kTileCells + e0) = make_double2(r[f][0], r[f][1]);
-    } else {
-      if (out0) {
-        ynew[o] = c[f][0];
-        K7g[o] = r[f][0];
-      }
-      if (out1) {
-        ynew[o + 1] = c[f][1];
-        K7g[o + 1] = r[f][1];
-      }
+    if (out0) {
+      ynew[o] = c[f][0];
+      K7g[o] = r[f][0];
+    }
+    if (out1) {
+      ynew[o + 1] = c[f][1];
+      K7g[o + 1] = r[f][1];
     }
     if (sample) {                                            // K3..K6 are only needed by the dense output
       if (out0) {
@@ -964,7 +807,6 @@ __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int p
     const unsigned bw = __reduce_or_sync(0xffffffffu, event_bits_sel(c, U, W, out0, out1));
     if ((tid & 31) == 0) reinterpret_cast<unsigned*>(red + kTileThreads / 32)[tid >> 5] = bw;
   }
-  if (TMA && tma) fence_proxy_async();                       // my staged values, for the bulk stores after the barrier
   __syncthreads();
   if (tid == 0) {
     double s = 0.0;
@@ -974,16 +816,6 @@ __global__ void __launch_bounds__(TT, 1) tile_attempt_kernel(const Args A, int p
       unsigned b = 0u;
       for (int w = 0; w < kTileThreads / 32; ++w) b |= reinterpret_cast<unsigned*>(red + kTileThreads / 32)[w];
       evpart_of(A, pin ^ 1, col)[tile] = b;
-    }
-    if (TMA && tma) {                                        // the cells this window owns: window positions [6, 2 TT - 6) inside the column
-      const int olo = w0 + kTileHalo, ohi = olo + kTileValid < N ? olo + kTileValid : N;
-      const unsigned bytes = (unsigned)(ohi - olo) * 8u;
-      const size_t row0 = (size_t)col * 5 * N + (size_t)olo;
-      for (int f = 0; f < 5; ++f) {
-        bulk_s2g(ynew + row0 + (size_t)f * N, sStage + f * kTileCells + kTileHalo, bytes);
-        bulk_s2g(K7g + row0 + (size_t)f * N, sStage + (5 + f) * kTileCells + kTileHalo, bytes);
-      }
-      bulk_commit_wait();
     }
   }
 }
@@ -996,12 +828,12 @@ namespace {
 struct GraphKey {             // everything a captured batch depends on (compared bytewise)
   st::Args a;
   long long attempts;
-  int use_tiles, device, small_tiles, tile_tma;
+  int device, small_tiles;
 };
 }  // namespace
 
-// the tile kernel instantiations: model variant x events x window size, plus the TMA-staged build of the plain one
-template <bool VD, bool EV, int TT, bool TMA>
+// the tile kernel instantiations: model variant x events x window size
+template <bool VD, bool EV, int TT>
 static cudaError_t tile_launch(const st::Args& a, unsigned tgrid, int cbuf, cudaStream_t s_) {
 #ifndef MARLPDE_HOST_EMU
   static bool configured = false;               // (per instantiation; the attribute is sticky per device context)
@@ -1009,24 +841,23 @@ static cudaError_t tile_launch(const st::Args& a, unsigned tgrid, int cbuf, cuda
   int dev = 0;
   cudaGetDevice(&dev);
   if (!configured || configured_device != dev) {
-    cudaError_t e = cudaFuncSetAttribute(st::tile_attempt_kernel<VD, EV, TT, TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)st::TileSmemT<TT, TMA>::total);
+    cudaError_t e = cudaFuncSetAttribute(st::tile_attempt_kernel<VD, EV, TT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)st::TileSmemT<TT>::total);
     if (e != cudaSuccess) return e;
     configured = true;
     configured_device = dev;
   }
 #endif
-  MARLPDE_LAUNCH((st::tile_attempt_kernel<VD, EV, TT, TMA>), tgrid, TT, (st::TileSmemT<TT, TMA>::total), s_, a, cbuf);
+  MARLPDE_LAUNCH((st::tile_attempt_kernel<VD, EV, TT>), tgrid, TT, (st::TileSmemT<TT>::total), s_, a, cbuf);
   return cudaSuccess;
 }
 
 template <int TT>
-static cudaError_t tile_dispatch(bool vd, bool ev, bool tma, const st::Args& a, unsigned tgrid, int cbuf, cudaStream_t s_) {
-  if (tma && !vd && !ev && TT == st::kTileThreadsLarge) return tile_launch<false, false, st::kTileThreadsLarge, true>(a, tgrid, cbuf, s_);
-  if (vd && ev) return tile_launch<true, true, TT, false>(a, tgrid, cbuf, s_);
-  if (vd) return tile_launch<true, false, TT, false>(a, tgrid, cbuf, s_);
-  if (ev) return tile_launch<false, true, TT, false>(a, tgrid, cbuf, s_);
-  return tile_launch<false, false, TT, false>(a, tgrid, cbuf, s_);
+static cudaError_t tile_dispatch(bool vd, bool ev, const st::Args& a, unsigned tgrid, int cbuf, cudaStream_t s_) {
+  if (vd && ev) return tile_launch<true, true, TT>(a, tgrid, cbuf, s_);
+  if (vd) return tile_launch<true, false, TT>(a, tgrid, cbuf, s_);
+  if (ev) return tile_launch<false, true, TT>(a, tgrid, cbuf, s_);
+  return tile_launch<false, false, TT>(a, tgrid, cbuf, s_);
 }
 
 cudaError_t launch_rk45_stream(double* d_y, const marlpde_column_params* d_params, marlpde_column_state* d_state,
@@ -1054,76 +885,55 @@ cudaError_t launch_rk45_stream(double* d_y, const marlpde_column_params* d_param
   a.tiles = (n_cells + st::kCellsPerCta - 1) / st::kCellsPerCta;
   a.pstride = (n_cells + 243) / 244 + 1;
   a.opt = opt;
-  a.tiles2 = 0;
   const long long blocks = (long long)a.tiles * n_columns;
   if (blocks > 0x7fffffffLL) return cudaErrorInvalidValue;
   const unsigned grid = (unsigned)blocks;
   const unsigned cgrid = (unsigned)((n_columns + 127) / 128);
-  // MARLPDE_RK45_STREAM=stages selects one launch per stage (HBM-streaming) instead of overlapped tiles
-  const char* mode_env = std::getenv("MARLPDE_RK45_STREAM");
-  const int use_tiles = (mode_env && mode_env[0] == 's') ? 0 : 1;
-  unsigned tgrid = 0;
-  // window size (MARLPDE_RK45_TILE=small|large overrides); MARLPDE_RK45_TILE_TMA=1 selects the TMA-staged build of the
-  // large window
-  bool small_tiles = false, tile_tma = false;
-  if (use_tiles) {
-    int sms = 148, dev = 0;
+  // window size (MARLPDE_RK45_TILE=small|large overrides)
+  int sms = 148, dev = 0;
 #ifndef MARLPDE_HOST_EMU
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
 #endif
-    const int valid_l = st::tile_valid_cells(st::kTileThreadsLarge), valid_s = st::tile_valid_cells(st::kTileThreadsSmall);
-    // small windows while ALL of them are resident at once (two 128-thread CTAs per SM: one wave at about two thirds
-    // of a large window's latency).  Measured (r02f, r02l; column-steps/s, small vs large): 20 000 x 1 49.6 k / 41.5 k,
-    // 20 000 x 3 130 k / 121 k, 5 000 x 12 567 k / 504 k, 2 000 x 32 1.53 M / 1.36 M — but 20 000 x 4 (328 small CTAs:
-    // two waves) 127 k / 160 k and 20 000 x 8 162 k / 176 k.
-    const long long ctas_small = (long long)((n_cells + valid_s - 1) / valid_s) * n_columns;
-    small_tiles = ctas_small <= 2LL * sms;
-    const char* tile_env = std::getenv("MARLPDE_RK45_TILE");
-    if (tile_env && tile_env[0] == 's') small_tiles = true;
-    if (tile_env && tile_env[0] == 'l') small_tiles = false;
-    const char* tma_env = std::getenv("MARLPDE_RK45_TILE_TMA");
-    tile_tma = tma_env && tma_env[0] == '1' && !small_tiles;
-    const int valid = small_tiles ? valid_s : valid_l;
-    a.tiles2 = (n_cells + valid - 1) / valid;
-    tgrid = (unsigned)((long long)a.tiles2 * n_columns);
-    (void)dev;
-  }
+  (void)dev;
+  const int valid_l = st::tile_valid_cells(st::kTileThreadsLarge), valid_s = st::tile_valid_cells(st::kTileThreadsSmall);
+  // small windows while ALL of them are resident at once (two 128-thread CTAs per SM: one wave at about two thirds
+  // of a large window's latency).  Measured (r02f, r02l; column-steps/s, small vs large): 20 000 x 1 49.6 k / 41.5 k,
+  // 20 000 x 3 130 k / 121 k, 5 000 x 12 567 k / 504 k, 2 000 x 32 1.53 M / 1.36 M — but 20 000 x 4 (328 small CTAs:
+  // two waves) 127 k / 160 k and 20 000 x 8 162 k / 176 k.
+  const long long ctas_small = (long long)((n_cells + valid_s - 1) / valid_s) * n_columns;
+  bool small_tiles = ctas_small <= 2LL * sms;
+  const char* tile_env = std::getenv("MARLPDE_RK45_TILE");
+  if (tile_env && tile_env[0] == 's') small_tiles = true;
+  if (tile_env && tile_env[0] == 'l') small_tiles = false;
+  const int valid = small_tiles ? valid_s : valid_l;
+  a.tiles2 = (n_cells + valid - 1) / valid;
+  const unsigned tgrid = (unsigned)((long long)a.tiles2 * n_columns);
   const bool var_dphi = (opt.flags & MARLPDE_FLAG_VAR_DPHI) != 0;
   const bool ev_on = (opt.flags & MARLPDE_FLAG_EVENTS) != 0;
-  // (the replay-and-locate protocol of prepare_kernel relies on the y ping-pong of the tile path: in the
-  //  one-launch-per-stage variant an accepted step overwrites y while another CTA would still read it)
-  if (ev_on && !use_tiles) return cudaErrorNotSupported;
   auto enqueue = [&](cudaStream_t s_) -> cudaError_t {
     MARLPDE_LAUNCH(st::init_kernel, cgrid, 128, 0, s_, a);
-    MARLPDE_LAUNCH(st::stage_kernel, grid, st::kThreads, 0, s_, a, 0, 0);            // K1 = f(y)
+    MARLPDE_LAUNCH(st::k1_kernel, grid, st::kThreads, 0, s_, a);
     int pin = 0;
-    // attempts + 1 prepares: the last one only closes the last attempt
+    // the tile kernel closes the previous attempt in its prologue: ONE launch per attempt; the prepare launch after the
+    // loop only closes the last attempt
     for (long long j = 0; j < attempts; ++j) {
-      if (use_tiles) {             // the tile kernel closes the previous attempt in its prologue: ONE launch per attempt
-        const cudaError_t et = small_tiles
-                                   ? tile_dispatch<st::kTileThreadsSmall>(var_dphi, ev_on, false, a, tgrid, pin, s_)
-                                   : tile_dispatch<st::kTileThreadsLarge>(var_dphi, ev_on, tile_tma, a, tgrid, pin, s_);
-        if (et != cudaSuccess) return et;
-      } else {
-        MARLPDE_LAUNCH(st::prepare_kernel, grid, st::kThreads, 0, s_, a, pin);
-        for (int i = 1; i <= 6; ++i) MARLPDE_LAUNCH(st::stage_kernel, grid, st::kThreads, 0, s_, a, i, pin ^ 1);
-      }
+      const cudaError_t et = small_tiles ? tile_dispatch<st::kTileThreadsSmall>(var_dphi, ev_on, a, tgrid, pin, s_)
+                                         : tile_dispatch<st::kTileThreadsLarge>(var_dphi, ev_on, a, tgrid, pin, s_);
+      if (et != cudaSuccess) return et;
       pin ^= 1;
     }
     MARLPDE_LAUNCH(st::prepare_kernel, grid, st::kThreads, 0, s_, a, pin);
     pin ^= 1;
-    if (use_tiles) MARLPDE_LAUNCH(st::copyback_kernel, grid, st::kThreads, 0, s_, a, pin);
+    MARLPDE_LAUNCH(st::copyback_kernel, grid, st::kThreads, 0, s_, a, pin);
     MARLPDE_LAUNCH(st::finish_kernel, cgrid, 128, 0, s_, a, pin);
     return cudaGetLastError();
   };
 #ifndef MARLPDE_HOST_EMU
   // The launches of a batch are captured once into a CUDA graph and replayed — a batch of a few columns is bound by launch
-  // latency (two dependent launches per attempt), and the host drivers repeat identical batches (all step state lives in
-  // device memory, the kernel arguments do not change).  Measured (r02a, profiles/r02a_ab_candidates.log): N = 20 000 x 1
-  // 37.3 -> 42.0 k attempts/s, N = 2 000 x 8 299 -> 353 k, N = 20 000 x 64 234.5 -> 238.3 k.  MARLPDE_RK45_STREAM_GRAPH=0
-  // launches kernel by kernel.
-  const char* graph_env = std::getenv("MARLPDE_RK45_STREAM_GRAPH");
-  if (!(graph_env && graph_env[0] == '0') && attempts <= 1024) {
+  // latency, and the host drivers repeat identical batches (all step state lives in device memory, the kernel arguments
+  // do not change).  Measured (r02a, profiles/r02a_ab_candidates.log): N = 20 000 x 1 37.3 -> 42.0 k attempts/s,
+  // N = 2 000 x 8 299 -> 353 k, N = 20 000 x 64 234.5 -> 238.3 k.
+  if (attempts <= 1024) {
     static std::mutex mu;
     static struct { bool valid; GraphKey key; cudaGraphExec_t exec; cudaStream_t cap; } cache = {false, {}, nullptr, nullptr};
     std::lock_guard<std::mutex> lock(mu);
@@ -1131,9 +941,7 @@ cudaError_t launch_rk45_stream(double* d_y, const marlpde_column_params* d_param
     std::memset(&key, 0, sizeof key);
     key.a = a;
     key.attempts = attempts;
-    key.use_tiles = use_tiles;
     key.small_tiles = small_tiles;
-    key.tile_tma = tile_tma;
     cudaError_t e = cudaGetDevice(&key.device);
     if (e != cudaSuccess) return e;
     if (!(cache.valid && std::memcmp(&cache.key, &key, sizeof key) == 0)) {

@@ -25,4 +25,4 @@ for i in range(3):
     torch.cuda.synchronize(); t0 = time.time()
     _cabi.check(lib.marlpde_rk45_stream_integrate_dev(y.data_ptr(), dP.data_ptr(), st.data_ptr(), B, N, C.byref(o), None, None, w.data_ptr(), nb, stream))
     torch.cuda.synchronize(); dt = time.time() - t0
-    print(f"call {i}: {att} attempts x {B} columns x {N} cells in {dt*1e3:.2f} ms -> {1680.0*N*B*att/dt/1e9:.0f} GB/s algorithmic, {B*att/dt:.3e} column-steps/s")
+    print(f"call {i}: {att} attempts x {B} columns x {N} cells in {dt*1e3:.2f} ms -> {160.0*N*B*att/dt/1e9:.0f} GB/s algorithmic, {B*att/dt:.3e} column-steps/s")

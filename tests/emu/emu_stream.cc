@@ -1,5 +1,5 @@
-// tests/emu/emu_stream.cc — the large-depth-grid RK45 path (csrc/rk45_streaming.cu: init / prepare / tile_attempt or stage
-// kernels / copyback / finish), compiled for the host; its own launcher runs unchanged, every launch executed block by
+// tests/emu/emu_stream.cc — the large-depth-grid RK45 path (csrc/rk45_streaming.cu: init / K1 / tile_attempt / prepare /
+// copyback / finish kernels), compiled for the host; its own launcher runs unchanged, every launch executed block by
 // block by the SIMT emulator.  TEST INFRASTRUCTURE ONLY (simt_emu.h).
 #include <cstdint>
 #include <vector>

@@ -328,10 +328,9 @@ def emu_stream():
     lib = C.CDLL(so)
     lib.emu_rk45_stream.restype = C.c_int
 
-    def run(P, y, t_end, t_eval, first_step, attempts, state=None, tma=0, events=False, counts=None, times=None, flags=0,
+    def run(P, y, t_end, t_eval, first_step, attempts, state=None, events=False, counts=None, times=None, flags=0,
             tile=None):
-        # the launcher reads its switches per call: TMA-staged windows, window size
-        os.environ["MARLPDE_RK45_TILE_TMA"] = "1" if tma else "0"
+        # the launcher reads the window size switch per call
         if tile:
             os.environ["MARLPDE_RK45_TILE"] = tile
         else:
@@ -354,11 +353,10 @@ def emu_stream():
 
 
 @pytest.mark.parametrize("n_cells,ncol", [(16, 2), (641, 2), (1257, 1)])
-def test_streaming_launcher_under_emulation_reproduces_scipy(emu_stream, n_cells, ncol, monkeypatch):
-    """csrc/rk45_streaming.cu with its own launcher (init / K1 / prepare + tile_attempt or six stage launches / copyback /
-    finish), every launch run block by block: both modes, ragged last tiles, batches of 16 attempts resumed from the
-    column state as the host driver does (csrc/cabi.cu rk45_integrate_streaming) — the GPU test
-    test_streaming_path_matches_scipy at a shorter t_end."""
+def test_streaming_launcher_under_emulation_reproduces_scipy(emu_stream, n_cells, ncol):
+    """csrc/rk45_streaming.cu with its own launcher (init / K1 / tile_attempt / prepare / copyback / finish), every launch
+    run block by block: ragged last windows, batches of 16 attempts resumed from the column state as the host driver
+    does (csrc/cabi.cu rk45_integrate_streaming) — the GPU test test_streaming_path_matches_scipy at a shorter t_end."""
     pde = oracle.default_scenario() | SCEN_A | {"N": n_cells}
     scale = min(1.0, (200 / n_cells) ** 2)
     t_end, fs = 60 * 2.6e-6 * scale, 1e-6 * scale
@@ -366,61 +364,51 @@ def test_streaming_launcher_under_emulation_reproduces_scipy(emu_stream, n_cells
     P, y0 = np.repeat(mb.derive_column_params(pde), ncol), np.repeat(mb.initial_state(pde), ncol, 0)
     sol = oracle.integrate(pde, method="RK45", t_span=(0, t_end), t_eval=te, events=False, first_step=fs)
     want = sol.y.reshape(5, n_cells, -1)
-    got = {}
-    for mode in ("tiles", "stages"):
-        monkeypatch.setenv("MARLPDE_RK45_STREAM", mode)
-        r = emu_stream(P, y0, t_end, te, fs, 16)
-        while np.any((r["state"]["status"] == 1) | (r["state"]["status"] == 2)):
-            nxt = emu_stream(P, r["y"], t_end, te, fs, 16, state=r["state"])
-            keep = np.isnan(nxt["snapshots"])
-            nxt["snapshots"][keep] = r["snapshots"][keep]
-            r = nxt
-        assert np.all(r["state"]["status"] == 0) and np.all(r["state"]["t"] == t_end) and np.all(r["state"]["next_eval"] == 3)
-        assert np.all(r["state"]["nfev"] == sol.nfev), (mode, r["state"]["nfev"], sol.nfev)
-        assert np.max(np.abs(r["y"][0] - want[:, :, -1])) <= 1e-12
-        assert np.max(np.abs(r["snapshots"][0] - np.moveaxis(want, 2, 0))) <= 1e-12
-        assert np.array_equal(r["y"][0], r["y"][-1])
-        got[mode] = r
-    for k in ("n_accepted", "n_rejected", "nfev"):
-        assert np.array_equal(got["tiles"]["state"][k], got["stages"]["state"][k]), k
-    assert np.max(np.abs(got["tiles"]["y"] - got["stages"]["y"])) <= 1e-12
+    r = emu_stream(P, y0, t_end, te, fs, 16)
+    while np.any((r["state"]["status"] == 1) | (r["state"]["status"] == 2)):
+        nxt = emu_stream(P, r["y"], t_end, te, fs, 16, state=r["state"])
+        keep = np.isnan(nxt["snapshots"])
+        nxt["snapshots"][keep] = r["snapshots"][keep]
+        r = nxt
+    assert np.all(r["state"]["status"] == 0) and np.all(r["state"]["t"] == t_end) and np.all(r["state"]["next_eval"] == 3)
+    assert np.all(r["state"]["nfev"] == sol.nfev), (r["state"]["nfev"], sol.nfev)
+    assert np.max(np.abs(r["y"][0] - want[:, :, -1])) <= 1e-12
+    assert np.max(np.abs(r["snapshots"][0] - np.moveaxis(want, 2, 0))) <= 1e-12
+    assert np.array_equal(r["y"][0], r["y"][-1])
 
 
 @pytest.mark.parametrize("n_cells", [16, 628, 1256, 1884, 1300])
-def test_tile_kernel_bulk_copy_windows_are_bit_identical(emu_stream, n_cells, monkeypatch):
-    """MARLPDE_RK45_TILE_TMA=1 (shipped, off by default: measured 10 % slower on B200): the tile kernel loads y and K1 of
-    its 640-cell window and stores y_new and K7 of the 628 cells it owns with ten 1-D bulk copies each way (on the host:
-    memcpy at issue).  Window clipping at both column ends, a column that ends exactly on a window boundary, one-window
-    columns and a sampled step: the same bits as the per-thread loads and stores.  Also the small windows (128 threads,
-    244 owned cells) a small batch is cut into."""
-    monkeypatch.setenv("MARLPDE_RK45_STREAM", "tiles")
+def test_tile_kernel_window_sizes_agree(emu_stream, n_cells):
+    """The tile kernel's two window sizes, each selected explicitly: 640-cell windows (320 threads, 628 owned cells) and
+    256-cell windows (128 threads, 244 owned cells).  Window clipping at both column ends, a column that ends exactly on
+    a window boundary, one-window columns and a sampled step.  The error norm adds one partial sum per window in window
+    order, so the step sizes of the two window sizes may differ in their last bits: same decisions, states equal to
+    round-off.  The launcher picks the small windows for every size here (one column on 148 SMs): bit for bit."""
     pde = oracle.default_scenario() | SCEN_A | {"N": n_cells}
     scale = min(1.0, (200 / n_cells) ** 2)
     fs = 1e-6 * scale
     te = [0.0, 4 * fs, 1.0]
     P, y0 = mb.derive_column_params(pde), mb.initial_state(pde)
     y0 = y0 * (1 + 0.01 * np.sin(np.arange(n_cells) * 0.37))          # a profile, so that misplaced rows would show
-    a = emu_stream(P, y0, 1.0, te, fs, 12)
-    b = emu_stream(P, y0, 1.0, te, fs, 12, tma=1)
-    assert a["state"]["n_accepted"][0] >= 8 and a["state"]["next_eval"][0] == 2
-    assert np.array_equal(a["state"], b["state"]) and np.array_equal(a["y"], b["y"])
-    assert np.array_equal(a["snapshots"][:, :2], b["snapshots"][:, :2])
-    # window size: the error norm adds one partial sum per window in window order, so the step sizes of the two window
-    # sizes may differ in their last bits — same decisions, states equal to round-off
-    c = emu_stream(P, y0, 1.0, te, fs, 12, tile="small")
+    large = emu_stream(P, y0, 1.0, te, fs, 12, tile="large")
+    small = emu_stream(P, y0, 1.0, te, fs, 12, tile="small")
+    auto = emu_stream(P, y0, 1.0, te, fs, 12)
+    assert large["state"]["n_accepted"][0] >= 8 and large["state"]["next_eval"][0] == 2
     for k in ("n_accepted", "n_rejected", "nfev", "status", "next_eval"):
-        assert np.array_equal(a["state"][k], c["state"][k]), k
-    assert abs(a["state"]["t"][0] - c["state"]["t"][0]) <= 1e-12 * a["state"]["t"][0]
-    assert np.max(np.abs(a["y"] - c["y"])) <= 1e-12 and np.max(np.abs(a["snapshots"][:, :2] - c["snapshots"][:, :2])) <= 1e-12
+        assert np.array_equal(large["state"][k], small["state"][k]), k
+    assert abs(large["state"]["t"][0] - small["state"]["t"][0]) <= 1e-12 * large["state"]["t"][0]
+    assert np.max(np.abs(large["y"] - small["y"])) <= 1e-12
+    assert np.max(np.abs(large["snapshots"][:, :2] - small["snapshots"][:, :2])) <= 1e-12
+    assert np.array_equal(auto["state"], small["state"]) and np.array_equal(auto["y"], small["y"])
+    assert np.array_equal(auto["snapshots"][:, :2], small["snapshots"][:, :2])
 
 
 @pytest.mark.parametrize("n_cells", [16, 1300])
-def test_streaming_events_replay_and_locate_under_emulation(emu_stream, n_cells, monkeypatch):
+def test_streaming_events_replay_and_locate_under_emulation(emu_stream, n_cells):
     """Event monitors on the streaming path: per-window predicate bits, detection in the prepare kernel, replay of the
     step with K3..K6 stored, Brent location by the column's first CTA.  Counts and root times equal SciPy's; a run cut
     into batches of 16 attempts (a batch may end between detection and location; 5 for the 16-cell grid) finds every event exactly once; the
     trajectory does not depend on monitoring."""
-    monkeypatch.setenv("MARLPDE_RK45_STREAM", "tiles")
     pde = oracle.default_scenario() | SCEN_A | {"N": n_cells}
     scale = min(1.0, (200 / n_cells) ** 2)
     t_end, fs = 90 * 2.6e-6 * scale, 1e-6 * scale

@@ -262,13 +262,17 @@ def test_events_survive_resume():
 
 
 # ---- depth grids that do not fit on chip: the streaming path (csrc/rk45_streaming.cu) ---------------
-@pytest.mark.parametrize("mode", ["tiles", "stages"])
+@pytest.mark.parametrize("window", ["auto", "large"])
 @pytest.mark.parametrize("n_cells,ncol", [(2000, 3), (5000, 1), (641, 2), (16, 2), (1257, 2)])
-def test_streaming_path_matches_scipy(n_cells, ncol, mode, monkeypatch):
+def test_streaming_path_matches_scipy(n_cells, ncol, window, monkeypatch):
     """BASELINE.json configs[3] (SURVEY.md §8d config 4): fixed budget of ~2000 steps, t_end and
     first_step scaled with (200/N)^2 (the explicit step is stability bound), state at t_end against SciPy
-    RK45 on the oracle.  Same stepper semantics as the on-chip kernel: nfev within two attempts."""
-    monkeypatch.setenv("MARLPDE_RK45_STREAM", mode)          # overlapped on-chip tiles (default) / one launch per stage
+    RK45 on the oracle.  Same stepper semantics as the on-chip kernel: nfev within two attempts.
+    window: the launcher's choice (256-cell windows for every batch here) or the 640-cell windows forced."""
+    if window == "large":
+        monkeypatch.setenv("MARLPDE_RK45_TILE", "large")
+    else:
+        monkeypatch.delenv("MARLPDE_RK45_TILE", raising=False)
     pde = oracle.default_scenario() | {"N": n_cells, "Phi0": 0.6, "PhiIni": 0.5, "PhiNR": 0.6}
     scale = min(1.0, (200 / n_cells) ** 2)
     t_end, fs = 600 * 2.6e-6 * scale, 1e-6 * scale
@@ -285,11 +289,9 @@ def test_streaming_path_matches_scipy(n_cells, ncol, mode, monkeypatch):
     assert np.array_equal(res.y[0], res.y[-1])
 
 
-def test_streaming_window_sizes_and_tma_staging_agree(monkeypatch):
-    """The tile kernel's builds: 640-cell windows (large batches), 256-cell windows (small batches, chosen by the launcher
-    when the large ones would leave more than half of the SMs idle) and the TMA-staged large window
-    (MARLPDE_RK45_TILE_TMA=1: UBLKCP bulk loads / stores through shared memory; shipped, off by default because it
-    measured 10 % slower).  TMA staging is bit-identical to the per-thread loads; the window size only changes the order
+def test_streaming_window_sizes_agree(monkeypatch):
+    """The tile kernel's two window sizes: 640-cell windows (large batches) and 256-cell windows (small batches, chosen by
+    the launcher when the large ones would leave more than half of the SMs idle).  The window size only changes the order
     in which the per-window error sums are added."""
     n_cells = 2000
     pde = oracle.default_scenario() | {"N": n_cells, "Phi0": 0.6, "PhiIni": 0.5, "PhiNR": 0.6}
@@ -298,15 +300,11 @@ def test_streaming_window_sizes_and_tma_staging_agree(monkeypatch):
     run = lambda: mb.integrate_rk45_batch(y0, P, t_span=(0, t_end), first_step=fs, t_eval=[0.5 * t_end, t_end])
     monkeypatch.setenv("MARLPDE_RK45_TILE", "large")
     large = run()
-    monkeypatch.setenv("MARLPDE_RK45_TILE_TMA", "1")
-    tma = run()
-    monkeypatch.delenv("MARLPDE_RK45_TILE_TMA")
     monkeypatch.setenv("MARLPDE_RK45_TILE", "small")
     small = run()
     monkeypatch.delenv("MARLPDE_RK45_TILE")
     auto = run()
     assert np.all(large.status == 0) and large.n_attempts[0] >= 200
-    assert np.array_equal(tma.y, large.y) and np.array_equal(tma.snapshots, large.snapshots) and np.array_equal(tma.nfev, large.nfev)
     assert np.array_equal(auto.y, small.y)                       # 3 columns x 4 large windows: the launcher picks small ones
     assert np.array_equal(small.nfev, large.nfev) and np.max(np.abs(small.y - large.y)) <= 1e-12
     assert np.max(np.abs(small.snapshots - large.snapshots)) <= 1e-12
