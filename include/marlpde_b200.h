@@ -282,6 +282,45 @@ int marlpde_bdf_integrate_async(double* y, const marlpde_column_params* params,
                                 double* snapshots, int32_t* event_counts, double* event_times,
                                 int64_t* stats, int device, void* stream);
 
+/* ---- forward parameter sensitivities on the BDF integrator (staggered direct method, sensitivities excluded from the
+ * error control; csrc/bdf_batch.cu, DESIGN.md 5.4) ------------------------------------------------------------------
+ *  For every column c and direction k < n_dirs (1 <= n_dirs <= 8) the kernel integrates s_k = dy/d eps_k,
+ *  s_k' = J(y) s_k + F_k(y), s_k(t0) = w_k, with the state's own step sequence: the same NDF formula, order, h and factors
+ *  after each accepted step.  The state's path (y, state, counters, snapshots, events) is bit-identical to
+ *  marlpde_bdf_integrate_dev's.  The derivative is taken at fixed nondimensional time t.
+ *  Arguments of marlpde_bdf_integrate_dev (opts->quantum must be 0), plus
+ *  d_params_pm  [n_columns][n_dirs][2]   the column's parameters moved by +sigma_k and by -sigma_k along direction k;
+ *               every integer field (FV_switch, mask_lo, mask_hi, model_flags) must equal the column's (checked: the
+ *               check synchronises `stream` once)
+ *  d_inv2sigma  [n_columns][n_dirs]      1 / (2 sigma_k): F_k = (f(y; p+) - f(y; p-)) inv2sigma
+ *  d_atol_s     [n_columns][n_dirs]      absolute tolerance of s_k in the corrector's convergence test (rtol: opts->rtol)
+ *  d_sens       [n_columns][n_dirs][5][n_cells]  in: w_k = s_k at state.t; out: s_k at the time reached (after
+ *               MARLPDE_STATUS_STEP_TOO_SMALL: at the last accepted step); a column resumed from a step budget passes it
+ *               back in and restarts at order 1, as the state does
+ *  d_sens_snap  [n_columns][n_dirs][n_eval][5][n_cells]  s_k at t_eval (may be NULL when n_eval == 0)
+ *  d_sens_stats [n_columns][3] int64, accumulated: corrector iterations, fallback factorisations of (I/c - J),
+ *               steps in which some direction did not converge
+ *  d_sens_workspace  marlpde_bdf_sens_workspace_bytes(n_columns, n_cells, n_dirs) bytes of device scratch
+ */
+size_t marlpde_bdf_sens_workspace_bytes(int n_columns, int n_cells, int n_dirs);
+int marlpde_bdf_sens_integrate_dev(double* d_y, const marlpde_column_params* d_params,
+                                   marlpde_column_state* d_state, int n_columns, int n_cells,
+                                   const marlpde_rk45_options* opts, const double* d_t_eval,
+                                   double* d_snapshots, int32_t* d_event_counts, double* d_event_times,
+                                   int64_t* d_stats, void* d_workspace, size_t workspace_bytes,
+                                   int32_t* d_queue, int n_dirs, const marlpde_column_params* d_params_pm,
+                                   const double* d_inv2sigma, const double* d_atol_s, double* d_sens,
+                                   double* d_sens_snap, int64_t* d_sens_stats, void* d_sens_workspace,
+                                   size_t sens_workspace_bytes, void* stream);
+/* host-pointer form: stages everything through pooled device scratch on one stream and synchronises */
+int marlpde_bdf_sens_integrate(double* y, const marlpde_column_params* params,
+                               marlpde_column_state* state, int n_columns, int n_cells,
+                               const marlpde_rk45_options* opts, const double* t_eval,
+                               double* snapshots, int32_t* event_counts, double* event_times,
+                               int64_t* stats, int n_dirs, const marlpde_column_params* params_pm,
+                               const double* inv2sigma, const double* atol_s, double* sens, double* sens_snap,
+                               int64_t* sens_stats, int device);
+
 /* ---- batched explicit Runge-Kutta integrators: Bogacki-Shampine RK23 and Dormand-Prince DOP853
  * (replace solve_ivp(method="RK23" | "DOP853") per column — marlpde/parameters.py:213; scipy/integrate/_ivp/rk.py —
  * step for step: same tableaux, step-size control, error norms and dense output, see csrc/erk_batch.cu) ------------

@@ -18,6 +18,13 @@
 // (they only precondition the iteration: the residual c f(y) - psi - d is fp64, and the error estimate is the converged
 // correction d itself, so — unlike Radau's — it carries no fp32 error).
 // A resumed column (step budget) restarts at order 1 from its stored state: the differences array is not kept.
+//
+// kSens = true adds forward parameter sensitivities s_k = dy/d eps_k (staggered direct method, DESIGN.md 5.4): after the
+// state's step is accepted every direction k takes the same NDF step for s_k' = J(y) s_k + F_k(y), with the step's order,
+// h, c and the state's factors; sensitivities never enter the error test, the order selection or the step size, so the
+// state's path is bit-identical with and without them.  kSens = false compiles to the kernel without sensitivities.
+#include <type_traits>
+
 #include "implicit_common.cuh"
 #include "bdf_batch.cuh"
 
@@ -160,13 +167,234 @@ __device__ __noinline__ bool rhs_residual(const ColumnConsts* kc, const fm::Tabl
   return __all_sync(0xffffffffu, finite);
 }
 
+// ---- forward sensitivities (kSens) ------------------------------------------------------------------------------------
+// Kernel arguments of the sensitivity build: the state's arguments plus, per column c and direction k < n_dirs,
+//   g_params_pm [B][P][2]   the column's parameters moved by +sigma_k / -sigma_k along direction k (host-derived)
+//   g_inv2sigma [B][P]      1 / (2 sigma_k): F_k = (f(y; p+) - f(y; p-)) inv2sigma
+//   g_atol_s    [B][P]      absolute tolerance of s_k in the corrector's convergence test
+//   g_sens      [B][P][5][N] in: s_k at the start time (w_k); out: s_k at the time reached (field-major like y)
+//   g_sens_snap [B][P][n_eval][5][N]  s_k at t_eval (field-major like the state's snapshots)
+//   g_sens_stats [B][3]     accumulated: corrector iterations, fallback factorisations, unconverged steps
+//   g_sens_work             sens_work_doubles(N, P) doubles per column
+struct SensArgs : Args {
+  const marlpde_column_params* g_params_pm;
+  const double* g_inv2sigma;
+  const double* g_atol_s;
+  double* g_sens;
+  double* g_sens_snap;
+  int64_t* g_sens_stats;
+  double* g_sens_work;
+  int n_dirs;
+};
+
+// per-column sensitivity workspace in doubles (n = 5 N), vectors CELL-major:
+//   J_s [N][3][5][5] (+N) | Rec_s [N][128] fp32 | per direction: D_s[8][n] | s[n] | psi_s[n] | d_s[n] | F[n]
+__host__ __device__ inline size_t sens_work_doubles(int N, int P) {
+  const size_t n = 5 * (size_t)N;
+  return 76 * (size_t)N + 64 * (size_t)N + (size_t)P * 12 * n;
+}
+
+// the perturbed constants of one warp (lane 0 derives them from p+ or p-; kSens builds only)
+__device__ __forceinline__ ColumnConsts* sens_consts(int warp) {
+  __shared__ ColumnConsts kc_pert[kWarpsPerCta];
+  return &kc_pert[warp];
+}
+
+// One RHS evaluation for the sensitivities: diff = false: out = f(yy); diff = true: out = (out - f(yy)) scale.
+template <bool VD>
+__device__ __noinline__ void sens_rhs(const ColumnConsts* kc, const fm::Tables* tb, int N, int lane, const double* yy,
+                                      double* out, bool diff, double scale, double (*stage)[2][kStageDoubles + 6]) {
+  auto sink = [&](int i, const double (&r5)[5]) {
+#pragma unroll
+    for (int f = 0; f < 5; ++f) out[i * 5 + f] = diff ? (out[i * 5 + f] - r5[f]) * scale : r5[f];
+  };
+  rhs_column<VD>(*kc, *tb, N, lane, yy, nullptr, stage, sink);
+  __syncwarp();
+}
+
+// fp64 block-tridiagonal mat-vec with the Jacobian blocks of jacobian(): out = a (J x + F) - m (p + q)  (p, q may be
+// NULL: then out = a (J x + F)).  One vector entry per lane and trip.
+__device__ __noinline__ void sens_matvec(int N, int lane, const double* J, const double* x, const double* F, double a,
+                                         double m, const double* p, const double* q, double* out) {
+  const int n = 5 * N;
+#pragma unroll 1
+  for (int idx = lane; idx < n; idx += 32) {
+    const int i = idx / 5, r = idx - 5 * i;
+    const double* blk = J + (size_t)i * 75;
+    double acc = F[idx];
+#pragma unroll
+    for (int f = 0; f < 5; ++f) acc = fma(blk[25 + f * 5 + r], x[i * 5 + f], acc);
+    if (i > 0) {
+#pragma unroll
+      for (int f = 0; f < 5; ++f) acc = fma(blk[f * 5 + r], x[(i - 1) * 5 + f], acc);
+    }
+    if (i < N - 1) {
+#pragma unroll
+      for (int f = 0; f < 5; ++f) acc = fma(blk[50 + f * 5 + r], x[(i + 1) * 5 + f], acc);
+    }
+    out[idx] = p ? fma(a, acc, -m * (p[idx] + q[idx])) : a * acc;
+  }
+  __syncwarp();
+}
+
+// Per-column view of the sensitivity workspace.
+struct SensCol {
+  double* Js;
+  float* Recs;
+  double* dirs;
+  size_t n;
+  __device__ double* D(int k) const { return dirs + (size_t)k * 12 * n; }
+  __device__ double* s(int k) const { return D(k) + 8 * n; }
+  __device__ double* psi(int k) const { return D(k) + 9 * n; }
+  __device__ double* d(int k) const { return D(k) + 10 * n; }
+  __device__ double* F(int k) const { return D(k) + 11 * n; }
+};
+
+// J_s = J(yy) (the kind the column's `jac` setting selects; the finite-difference kind needs f = f(yy) with the column's
+// own constants: given, or formed in ftmp when f is NULL) and F_k(yy) of every direction.  Nothing of the state is
+// touched: `scratch` (2 n) is the state's Jacobian scratch and `ftmp` (n) its tmp vector, both dead between steps.
+template <bool VD, bool kJacFD>
+__device__ __forceinline__ void sens_prepare(WarpScratch& ws, const ColumnConsts& kc, const fm::Tables& tb, int N, int lane,
+                                          const SensArgs& A, int col, const SensCol& sc, const double* yy,
+                                          const double* f, double* ftmp, double* scratch) {
+  if (kJacFD && !f) {
+    sens_rhs<VD>(&kc, &tb, N, lane, yy, ftmp, false, 1.0, ws.stage);
+    f = ftmp;
+  }
+  imp::jacobian<VD, kJacFD>(kc, tb, N, lane, yy, f, A.opt.atol, sc.Js, scratch, ws.stage);
+  ColumnConsts* const kp = sens_consts(threadIdx.x >> 5);
+#pragma unroll 1
+  for (int k = 0; k < A.n_dirs; ++k) {
+    const marlpde_column_params* pm = A.g_params_pm + ((size_t)col * A.n_dirs + k) * 2;
+    if (lane == 0) make_consts(pm[0], N, *kp);
+    __syncwarp();
+    sens_rhs<VD>(kp, &tb, N, lane, yy, sc.F(k), false, 1.0, ws.stage);
+    if (lane == 0) make_consts(pm[1], N, *kp);
+    __syncwarp();
+    sens_rhs<VD>(kp, &tb, N, lane, yy, sc.F(k), true, A.g_inv2sigma[(size_t)col * A.n_dirs + k], ws.stage);
+  }
+}
+
+// The sensitivity corrector of one accepted step (order, c; the state's factors Rec hold M_lu I - J_old).  Per direction:
+// s_pred = sum D_s[0..order], psi_s = D_s[1..order]^T gamma / alpha, then d_s = c (J_s s + F) - psi_s solved by the
+// state's simplified Newton iteration on its own (stale) factors; if that does not converge, (I/c - J_s) is factorised
+// into Rec_s once per step and the iteration restarts from the predictor; a direction that still fails keeps its last
+// iterate and the step is counted as unconverged.  Leaves s_new in s, the converged correction in d_s.  `b` (n) is the
+// state's right-hand-side buffer, dead between steps.
+__device__ __noinline__ void sens_correct(WarpScratch& ws, int N, int lane, const SensArgs& A, int col, const SensCol& sc,
+                                          int order, double c, double M_lu, const float* Rec, double newton_tol,
+                                          double* b, long long& n_iter, long long& n_fact, long long& n_unconv) {
+  const int n = 5 * N;
+  const double rtol = A.opt.rtol;
+  const double ia = 1.0 / kAlpha[order];
+  bool factored = false, unconverged = false;
+#pragma unroll 1
+  for (int k = 0; k < A.n_dirs; ++k) {
+    double* const Ds = sc.D(k);
+    double* const s = sc.s(k);
+    double* const psi = sc.psi(k);
+    double* const d = sc.d(k);
+    const double atol_s = A.g_atol_s[(size_t)col * A.n_dirs + k];
+    auto predict = [&]() {
+#pragma unroll 1
+      for (int idx = lane; idx < n; idx += 32) {
+        double v = Ds[idx], ps = 0.0;
+#pragma unroll
+        for (int j = 1; j <= kMaxOrder; ++j)
+          if (j <= order) {
+            const double x = Ds[(size_t)j * n + idx];
+            v += x;
+            ps = fma(x, kGamma[j], ps);
+          }
+        s[idx] = v;
+        psi[idx] = ps * ia;
+        d[idx] = 0.0;
+      }
+      __syncwarp();
+    };
+    // the state's iteration and rate test (solve_bdf_system), scale atol_s + rtol |s_pred|
+    auto iterate = [&](const float* R, double Mlu) -> bool {
+      const double Mc = Mlu * c;
+      double norm_old = -1.0;
+#pragma unroll 1
+      for (int it = 0; it < kNewtonMaxIter; ++it) {
+        sens_matvec(N, lane, sc.Js, s, sc.F(k), Mc, Mlu, psi, d, b);
+        solve<true>(ws, N, lane, R, b, nullptr, nullptr, false);
+        double ss = 0.0;
+#pragma unroll 1
+        for (int idx = lane; idx < n; idx += 32) {
+          const double dx = b[idx], sv = s[idx], dv = d[idx];
+          const double a = dx / fma(fabs(sv - dv), rtol, atol_s);
+          ss = fma(a, a, ss);
+          s[idx] = sv + dx;
+          d[idx] = dv + dx;
+        }
+        __syncwarp();
+        n_iter += 1;
+        const double norm = sqrt(warp_sum(ss) / (double)n);
+        const double rate = norm_old >= 0.0 ? norm / norm_old : -1.0;
+        double rate_pow = rate;
+        for (int e = 1; e < kNewtonMaxIter - it; ++e) rate_pow *= rate;
+        if (!(norm == norm)) return false;
+        if (rate >= 0.0 && (rate >= 1.0 || rate_pow / (1.0 - rate) * norm > newton_tol)) return false;
+        if (norm == 0.0 || (rate >= 0.0 && rate / (1.0 - rate) * norm < newton_tol)) return true;
+        norm_old = norm;
+      }
+      return false;
+    };
+    predict();
+    if (iterate(Rec, M_lu)) continue;
+    if (!factored) {
+      factorise<false>(ws, N, lane, 1.0 / c, make_double2(0.0, 0.0), sc.Js, sc.Recs);
+      factored = true;
+      n_fact += 1;
+    }
+    predict();
+    if (!iterate(sc.Recs, 1.0 / c)) unconverged = true;
+  }
+  if (unconverged) n_unconv += 1;
+}
+
+// bdf.py's post-acceptance update of the differences, applied to every D_s: D[order+2] = d - D[order+1],
+// D[order+1] = d, D[i] += D[i+1] for i = order .. 0
+__device__ __noinline__ void sens_update_D(int N, int lane, const SensCol& sc, int P, int order) {
+  const int n = 5 * N;
+#pragma unroll 1
+  for (int k = 0; k < P; ++k) {
+    double* const D = sc.D(k);
+    const double* const d = sc.d(k);
+#pragma unroll 1
+    for (int idx = lane; idx < n; idx += 32) {
+      const double dv = d[idx];
+      D[(size_t)(order + 2) * n + idx] = dv - D[(size_t)(order + 1) * n + idx];
+      D[(size_t)(order + 1) * n + idx] = dv;
+      double run = dv;
+#pragma unroll
+      for (int i = kMaxOrder; i >= 0; --i)
+        if (i <= order) {
+          run += D[(size_t)i * n + idx];
+          D[(size_t)i * n + idx] = run;
+        }
+    }
+  }
+  __syncwarp();
+}
+
+// every change_D of the state is applied with the same factor to every D_s
+__device__ __noinline__ void sens_change_D(WarpScratch& ws, int n, int lane, const SensCol& sc, int P, int order,
+                                           double factor) {
+#pragma unroll 1
+  for (int k = 0; k < P; ++k) change_D(ws, n, lane, sc.D(k), order, factor);
+}
+
 // resident CTAs per SM (r02v, 4096 / 64 lattice columns to t = 0.05): 2 -> 2.40 / 0.73 s, 3 -> 1.90 / 0.75 s, 4 -> 1.83 / 0.84 s
 #ifndef MARLPDE_BDF_MINBLOCKS
 #define MARLPDE_BDF_MINBLOCKS 3
 #endif
 
-template <bool VD, bool kJacFD>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_kernel(const Args A) {
+template <bool VD, bool kJacFD, bool kSens = false>
+__global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS)
+    bdf_kernel(const std::conditional_t<kSens, SensArgs, Args> A) {
   __shared__ __align__(16) unsigned char tab_raw[fm::kTableBytes];
   __shared__ WarpScratch scratch[kWarpsPerCta];
   const fm::Tables tb = fm::stage_tables(tab_raw, threadIdx.x, blockDim.x);
@@ -211,6 +439,29 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
     long long n_acc = st.n_accepted, n_rej = st.n_rejected, nfev = st.nfev;
     long long njev = 0, nlu = 0, n_newton = 0, n_newton_fail = 0;
     int next_eval = st.next_eval;
+    SensCol sc{};                                        // kSens: this column's sensitivity workspace
+    long long s_iter = 0, s_fact = 0, s_unconv = 0;
+    const double t_start = st.t;
+    if constexpr (kSens) {
+      double* sb = A.g_sens_work + (size_t)col * sens_work_doubles(N, A.n_dirs);
+      sc.Js = sb;
+      sc.Recs = reinterpret_cast<float*>(sb + 76 * (size_t)N);
+      sc.dirs = sb + 140 * (size_t)N;
+      sc.n = (size_t)n;
+#pragma unroll 1
+      for (int k = 0; k < A.n_dirs; ++k) {
+        const double* w = A.g_sens + ((size_t)col * A.n_dirs + k) * n;
+        double* const Ds = sc.D(k);
+        double* const s = sc.s(k);
+#pragma unroll 1
+        for (int idx = lane; idx < n; idx += 32) {
+          const double v = w[(idx % 5) * N + idx / 5];
+          s[idx] = v;
+          Ds[idx] = v;
+        }
+      }
+      __syncwarp();
+    }
     int status = MARLPDE_STATUS_FINISHED;
     long long steps_done = 0;
     int order = 1, n_equal_steps = 0;
@@ -236,6 +487,12 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
 #pragma unroll 1
       for (int idx = lane; idx < n; idx += 32) D[(size_t)n + idx] = f[idx] * h_abs;   // D[1] = f h
       __syncwarp();
+      if constexpr (kSens) {                             // D_s[1] = h (J(y0) w + F(y0))
+        sens_prepare<VD, kJacFD>(ws, kc, tb, N, lane, A, col, sc, y, f, tmp, jscr);
+#pragma unroll 1
+        for (int k = 0; k < A.n_dirs; ++k)
+          sens_matvec(N, lane, sc.Js, sc.s(k), sc.F(k), h_abs, 0.0, nullptr, nullptr, sc.D(k) + n);
+      }
     }
     const bool ev_on = (A.opt.flags & MARLPDE_FLAG_EVENTS) != 0;
     unsigned ev_prev = 0u;
@@ -250,10 +507,12 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
       const double min_step = 10.0 * (__longlong_as_double(__double_as_longlong(t) + 1) - t);
       if (h_abs > A.opt.max_step) {
         change_D(ws, n, lane, D, order, A.opt.max_step / h_abs);
+        if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, A.opt.max_step / h_abs);
         h_abs = A.opt.max_step;
         n_equal_steps = 0;
       } else if (h_abs < min_step) {
         change_D(ws, n, lane, D, order, min_step / h_abs);
+        if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, min_step / h_abs);
         h_abs = min_step;
         n_equal_steps = 0;
       }
@@ -270,6 +529,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
         if (t_new - A.opt.t_bound > 0.0) {
           t_new = A.opt.t_bound;
           change_D(ws, n, lane, D, order, fabs(t_new - t) / h_abs);
+          if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, fabs(t_new - t) / h_abs);
           n_equal_steps = 0;
           lu_valid = false;
         }
@@ -364,6 +624,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
         if (!converged) {
           h_abs *= 0.5;
           change_D(ws, n, lane, D, order, 0.5);
+          if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, 0.5);
           n_equal_steps = 0;
           lu_valid = false;
           continue;
@@ -382,6 +643,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
           const double factor = fmax(kMinFactor, safety * pow(error_norm, -1.0 / (double)(order + 1)));
           h_abs *= factor;
           change_D(ws, n, lane, D, order, factor);
+          if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, factor);
           n_equal_steps = 0;
           n_rej += 1;                                    // (no trouble with convergence: the factors are kept)
         } else {
@@ -391,6 +653,12 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
       if (failed) {
         status = MARLPDE_STATUS_STEP_TOO_SMALL;
         break;
+      }
+      if constexpr (kSens) {                             // the sensitivities' step with this step's order, h, c, factors
+        sens_prepare<VD, kJacFD>(ws, kc, tb, N, lane, A, col, sc, y, nullptr, tmp, jscr);
+        sens_correct(ws, N, lane, A, col, sc, order, (t_new - t) / kAlpha[order], M_lu, Rec, newton_tol, b, s_iter,
+                     s_fact, s_unconv);
+        sens_update_D(N, lane, sc, A.n_dirs, order);
       }
       // ------------------------------------------------------------------ accepted step
       n_equal_steps += 1;
@@ -443,6 +711,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
         const double factor = fmin(kMaxFactor, safety * best);
         h_abs *= factor;
         change_D(ws, n, lane, D, order, factor);
+        if constexpr (kSens) sens_change_D(ws, n, lane, sc, A.n_dirs, order, factor);
         n_equal_steps = 0;
         lu_valid = false;
       }
@@ -465,6 +734,18 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
         double* snap = A.g_snap + ((size_t)col * A.opt.n_eval + next_eval) * n;
         _Pragma("unroll 1") for (int idx = lane; idx < n; idx += 32)
           snap[(idx % 5) * N + idx / 5] = dense_value(D, n, idx, order, p);
+        if constexpr (kSens) {                           // (a sample at the start time is w itself)
+#pragma unroll 1
+          for (int k = 0; k < A.n_dirs; ++k) {
+            const double* w = A.g_sens + ((size_t)col * A.n_dirs + k) * n;
+            double* ss = A.g_sens_snap + (((size_t)col * A.n_dirs + k) * A.opt.n_eval + next_eval) * n;
+            const double* Ds = sc.D(k);
+            _Pragma("unroll 1") for (int idx = lane; idx < n; idx += 32) {
+              const int fi = (idx % 5) * N + idx / 5;
+              ss[fi] = te == t_start ? w[fi] : dense_value(Ds, n, idx, order, p);
+            }
+          }
+        }
         ++next_eval;
       }
     }
@@ -473,6 +754,22 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MARLPDE_BDF_MINBLOCKS) bdf_
     const double* const y_out = status == MARLPDE_STATUS_STEP_TOO_SMALL ? D : y;
 #pragma unroll 1
     for (int idx = lane; idx < n; idx += 32) gy[(idx % 5) * N + idx / 5] = y_out[idx];
+    if constexpr (kSens) {                               // s at time t, mirroring y_out (w is read above: sync first)
+      __syncwarp();
+#pragma unroll 1
+      for (int k = 0; k < A.n_dirs; ++k) {
+        const double* s_out = status == MARLPDE_STATUS_STEP_TOO_SMALL ? sc.D(k) : sc.s(k);
+        double* gs = A.g_sens + ((size_t)col * A.n_dirs + k) * n;
+#pragma unroll 1
+        for (int idx = lane; idx < n; idx += 32) gs[(idx % 5) * N + idx / 5] = s_out[idx];
+      }
+      if (lane == 0) {
+        int64_t* s3 = A.g_sens_stats + (size_t)col * 3;
+        s3[0] += s_iter;
+        s3[1] += s_fact;
+        s3[2] += s_unconv;
+      }
+    }
     if (lane == 0) {
       st.t = t;
       st.h_abs = h_abs;
@@ -527,6 +824,75 @@ cudaError_t launch_bdf(double* d_y, const marlpde_column_params* d_params, marlp
   else if (vd) bd::bdf_kernel<true, false><<<ctas, threads, 0, stream>>>(a);
   else if (fd) bd::bdf_kernel<false, true><<<ctas, threads, 0, stream>>>(a);
   else bd::bdf_kernel<false, false><<<ctas, threads, 0, stream>>>(a);
+  return cudaGetLastError();
+}
+#endif
+
+size_t bdf_sens_workspace_bytes(int n_columns, int n_cells, int n_dirs) {
+  return sizeof(double) * bd::sens_work_doubles(n_cells, n_dirs) * (size_t)n_columns;
+}
+
+#ifndef MARLPDE_HOST_EMU
+namespace bd {
+// bad[0] += number of (column, direction, sign) whose perturbed parameters differ from the column's in an integer field
+__global__ void sens_check_kernel(const marlpde_column_params* p, const marlpde_column_params* pm, int n_columns,
+                                  int n_dirs, int32_t* bad) {
+  const long long total = 2LL * n_columns * n_dirs;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const marlpde_column_params& a = p[e / (2 * n_dirs)];
+    const marlpde_column_params& q = pm[e];
+    if (a.FV_switch != q.FV_switch || a.mask_lo != q.mask_lo || a.mask_hi != q.mask_hi || a.model_flags != q.model_flags)
+      atomicAdd(bad, 1);
+  }
+}
+}  // namespace bd
+
+cudaError_t launch_bdf_sens_check(const marlpde_column_params* d_params, const marlpde_column_params* d_params_pm,
+                                  int n_columns, int n_dirs, int32_t* d_bad, cudaStream_t stream) {
+  const long long total = 2LL * n_columns * n_dirs;
+  const int blocks = (int)((total + 255) / 256 < 1024 ? (total + 255) / 256 : 1024);
+  bd::sens_check_kernel<<<blocks > 0 ? blocks : 1, 256, 0, stream>>>(d_params, d_params_pm, n_columns, n_dirs, d_bad);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_bdf_sens(double* d_y, const marlpde_column_params* d_params, marlpde_column_state* d_state,
+                            int n_columns, int n_cells, const marlpde_rk45_options& opt, const double* d_t_eval,
+                            double* d_snap, int64_t* d_stats, int32_t* d_ev_counts, double* d_ev_times, double* d_work,
+                            int32_t* d_queue, int n_dirs, const marlpde_column_params* d_params_pm,
+                            const double* d_inv2sigma, const double* d_atol_s, double* d_sens, double* d_sens_snap,
+                            int64_t* d_sens_stats, double* d_sens_work, int sm_count, cudaStream_t stream) {
+  bd::SensArgs a;
+  a.g_y = d_y;
+  a.g_params = d_params;
+  a.g_state = d_state;
+  a.g_t_eval = d_t_eval;
+  a.g_snap = d_snap;
+  a.g_stats = d_stats;
+  a.g_ev_counts = d_ev_counts;
+  a.g_ev_times = d_ev_times;
+  a.g_work = d_work;
+  a.g_queue = d_queue;
+  a.n_columns = n_columns;
+  a.N = n_cells;
+  a.opt = opt;
+  a.g_params_pm = d_params_pm;
+  a.g_inv2sigma = d_inv2sigma;
+  a.g_atol_s = d_atol_s;
+  a.g_sens = d_sens;
+  a.g_sens_snap = d_sens_snap;
+  a.g_sens_stats = d_sens_stats;
+  a.g_sens_work = d_sens_work;
+  a.n_dirs = n_dirs;
+  int ctas = (n_columns + imp::kWarpsPerCta - 1) / imp::kWarpsPerCta;
+  const int max_ctas = sm_count * MARLPDE_BDF_MINBLOCKS;
+  if (ctas > max_ctas) ctas = max_ctas;
+  if (ctas < 1) ctas = 1;
+  const bool vd = (opt.flags & MARLPDE_FLAG_VAR_DPHI) != 0, fd = (opt.flags & MARLPDE_FLAG_JAC_FD) != 0;
+  const int threads = imp::kWarpsPerCta * 32;
+  if (vd && fd) bd::bdf_kernel<true, true, true><<<ctas, threads, 0, stream>>>(a);
+  else if (vd) bd::bdf_kernel<true, false, true><<<ctas, threads, 0, stream>>>(a);
+  else if (fd) bd::bdf_kernel<false, true, true><<<ctas, threads, 0, stream>>>(a);
+  else bd::bdf_kernel<false, false, true><<<ctas, threads, 0, stream>>>(a);
   return cudaGetLastError();
 }
 #endif

@@ -658,6 +658,169 @@ int marlpde_bdf_integrate_async(double* y, const marlpde_column_params* params, 
                                  event_times, stats, device, (cudaStream_t)stream, false);
 }
 
+// ---- forward sensitivities on the BDF integrator: the BDF arguments and checks plus the per-direction buffers ---------
+size_t marlpde_bdf_sens_workspace_bytes(int n_columns, int n_cells, int n_dirs) {
+  if (n_columns <= 0 || n_cells <= 0 || n_dirs <= 0) return 0;
+  return marlpde::bdf_sens_workspace_bytes(n_columns, n_cells, n_dirs);
+}
+
+static int check_sens_args(int n_dirs) {
+  if (n_dirs < 1 || n_dirs > marlpde::kBdfMaxDirs)
+    return fail(MARLPDE_EINVAL, "n_dirs must be in [1, %d] (got %d)", marlpde::kBdfMaxDirs, n_dirs);
+  return MARLPDE_OK;
+}
+
+static int sens_field_mismatch(int n_bad) {
+  return fail(MARLPDE_EINVAL, "%d perturbed parameter sets differ from their column's in an integer field (FV_switch, "
+              "mask_lo, mask_hi or model_flags): a direction moved a mask boundary or a switch, where the state does "
+              "not depend smoothly on the parameter", n_bad);
+}
+
+int marlpde_bdf_sens_integrate_dev(double* d_y, const marlpde_column_params* d_params, marlpde_column_state* d_state,
+                                   int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* d_t_eval,
+                                   double* d_snapshots, int32_t* d_event_counts, double* d_event_times, int64_t* d_stats,
+                                   void* d_workspace, size_t workspace_bytes, int32_t* d_queue, int n_dirs,
+                                   const marlpde_column_params* d_params_pm, const double* d_inv2sigma,
+                                   const double* d_atol_s, double* d_sens, double* d_sens_snap, int64_t* d_sens_stats,
+                                   void* d_sens_workspace, size_t sens_workspace_bytes, void* stream) {
+  int rc = check_implicit_args(n_columns, n_cells, opts);
+  if (rc) return rc;
+  rc = check_sens_args(n_dirs);
+  if (rc) return rc;
+  if (n_columns == 0) return MARLPDE_OK;
+  if (!d_y || !d_params || !d_state || !d_queue || !d_stats || !d_workspace)
+    return fail(MARLPDE_EINVAL, "NULL device pointer");
+  if (!d_params_pm || !d_inv2sigma || !d_atol_s || !d_sens || !d_sens_stats || !d_sens_workspace)
+    return fail(MARLPDE_EINVAL, "NULL sensitivity pointer");
+  if (opts->n_eval > 0 && (!d_t_eval || !d_snapshots || !d_sens_snap))
+    return fail(MARLPDE_EINVAL, "n_eval > 0 needs t_eval, snapshots and sensitivity snapshots");
+  if (opts->flags & MARLPDE_FLAG_EVENTS) {
+    if (!d_event_counts) return fail(MARLPDE_EINVAL, "MARLPDE_FLAG_EVENTS needs event_counts");
+    if (opts->event_capacity > 0 && !d_event_times) return fail(MARLPDE_EINVAL, "event_capacity > 0 needs event_times");
+  }
+  if (opts->quantum != 0) return fail(MARLPDE_EUNSUPPORTED, "team columns (opts->quantum) are a Radau feature");
+  const size_t need = marlpde::bdf_workspace_bytes(n_columns, n_cells);
+  if (workspace_bytes < need) return fail(MARLPDE_EINVAL, "workspace too small: %zu < %zu bytes", workspace_bytes, need);
+  const size_t need_s = marlpde::bdf_sens_workspace_bytes(n_columns, n_cells, n_dirs);
+  if (sens_workspace_bytes < need_s)
+    return fail(MARLPDE_EINVAL, "sensitivity workspace too small: %zu < %zu bytes", sens_workspace_bytes, need_s);
+  DevProps props;
+  rc = current_props(props);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  {  // integer fields of p+ / p- against the column's: one small kernel, one 4-byte read-back
+    DevBuf bad;
+    CU(bad.alloc(sizeof(int32_t), s));
+    CU(cudaMemsetAsync(bad.p, 0, sizeof(int32_t), s));
+    CU(marlpde::launch_bdf_sens_check(d_params, d_params_pm, n_columns, n_dirs, bad.as<int32_t>(), s));
+    int32_t n_bad = 0;
+    CU(cudaMemcpyAsync(&n_bad, bad.p, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (n_bad) return sens_field_mismatch(n_bad);
+  }
+  cudaError_t e = marlpde::launch_bdf_sens(d_y, d_params, d_state, n_columns, n_cells, *opts, d_t_eval, d_snapshots,
+                                           d_stats, d_event_counts, d_event_times, static_cast<double*>(d_workspace),
+                                           d_queue, n_dirs, d_params_pm, d_inv2sigma, d_atol_s, d_sens, d_sens_snap,
+                                           d_sens_stats, static_cast<double*>(d_sens_workspace), props.sm_count, s);
+  if (e != cudaSuccess) return cuda_fail(e, "bdf sensitivity launch");
+  return MARLPDE_OK;
+}
+
+int marlpde_bdf_sens_integrate(double* y, const marlpde_column_params* params, marlpde_column_state* state,
+                               int n_columns, int n_cells, const marlpde_rk45_options* opts, const double* t_eval,
+                               double* snapshots, int32_t* event_counts, double* event_times, int64_t* stats,
+                               int n_dirs, const marlpde_column_params* params_pm, const double* inv2sigma,
+                               const double* atol_s, double* sens, double* sens_snap, int64_t* sens_stats, int device) {
+  int rc = check_implicit_args(n_columns, n_cells, opts);
+  if (rc) return rc;
+  rc = check_sens_args(n_dirs);
+  if (rc) return rc;
+  if (n_columns == 0) return MARLPDE_OK;
+  if (!y || !params || !state || !stats) return fail(MARLPDE_EINVAL, "NULL pointer");
+  if (!params_pm || !inv2sigma || !atol_s || !sens || !sens_stats) return fail(MARLPDE_EINVAL, "NULL sensitivity pointer");
+  if (opts->n_eval > 0 && (!t_eval || !snapshots || !sens_snap))
+    return fail(MARLPDE_EINVAL, "n_eval > 0 needs t_eval, snapshots and sensitivity snapshots");
+  int n_bad = 0;
+  for (int c = 0; c < n_columns; ++c)
+    for (int k = 0; k < 2 * n_dirs; ++k) {
+      const marlpde_column_params &a = params[c], &q = params_pm[(size_t)c * 2 * n_dirs + k];
+      n_bad += a.FV_switch != q.FV_switch || a.mask_lo != q.mask_lo || a.mask_hi != q.mask_hi ||
+               a.model_flags != q.model_flags;
+    }
+  if (n_bad) return sens_field_mismatch(n_bad);
+  DeviceScope scope;
+  rc = scope.enter(device);
+  if (rc) return rc;
+  cudaStream_t s = cudaStreamPerThread;
+  const size_t P = (size_t)n_dirs;
+  const size_t nb_y = sizeof(double) * 5 * (size_t)n_cells * n_columns;
+  const size_t nb_snap = nb_y * (size_t)opts->n_eval;
+  const size_t nb_p = sizeof(marlpde_column_params) * (size_t)n_columns;
+  const size_t nb_s = sizeof(marlpde_column_state) * (size_t)n_columns;
+  const size_t nb_stats = sizeof(int64_t) * 4 * (size_t)n_columns;
+  const size_t nb_work = marlpde::bdf_workspace_bytes(n_columns, n_cells);
+  const size_t nb_ec = sizeof(int32_t) * MARLPDE_NEVENTS * (size_t)n_columns;
+  const size_t nb_et = sizeof(double) * MARLPDE_NEVENTS * (size_t)(opts->event_capacity > 0 ? opts->event_capacity : 0) * n_columns;
+  const size_t nb_pm = 2 * P * nb_p, nb_dir = sizeof(double) * P * (size_t)n_columns;
+  const size_t nb_sens = P * nb_y, nb_ssnap = P * nb_snap, nb_sstats = sizeof(int64_t) * 3 * (size_t)n_columns;
+  const size_t nb_swork = marlpde::bdf_sens_workspace_bytes(n_columns, n_cells, n_dirs);
+  DevBuf dy, dp, ds, dte, dsnap, dq, dst, dw, dec, det, dpm, dis, dat, dsens, dssnap, dsst, dsw;
+  CU(dec.alloc(nb_ec, s));
+  CU(det.alloc(nb_et, s));
+  if (event_counts) CU(cudaMemcpyAsync(dec.p, event_counts, nb_ec, cudaMemcpyHostToDevice, s));
+  else CU(cudaMemsetAsync(dec.p, 0, nb_ec, s));
+  if (event_times && nb_et) CU(cudaMemcpyAsync(det.p, event_times, nb_et, cudaMemcpyHostToDevice, s));
+  CU(dy.alloc(nb_y, s));
+  CU(dp.alloc(nb_p, s));
+  CU(ds.alloc(nb_s, s));
+  CU(dte.alloc(sizeof(double) * (size_t)opts->n_eval, s));
+  CU(dsnap.alloc(nb_snap, s));
+  CU(dq.alloc(sizeof(int32_t), s));
+  CU(dst.alloc(nb_stats, s));
+  CU(dw.alloc(nb_work, s));
+  CU(dpm.alloc(nb_pm, s));
+  CU(dis.alloc(nb_dir, s));
+  CU(dat.alloc(nb_dir, s));
+  CU(dsens.alloc(nb_sens, s));
+  CU(dssnap.alloc(nb_ssnap, s));
+  CU(dsst.alloc(nb_sstats, s));
+  CU(dsw.alloc(nb_swork, s));
+  CU(cudaMemcpyAsync(dy.p, y, nb_y, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dp.p, params, nb_p, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(ds.p, state, nb_s, cudaMemcpyHostToDevice, s));
+  if (opts->n_eval) CU(cudaMemcpyAsync(dte.p, t_eval, sizeof(double) * (size_t)opts->n_eval, cudaMemcpyHostToDevice, s));
+  if (snapshots && nb_snap) CU(cudaMemcpyAsync(dsnap.p, snapshots, nb_snap, cudaMemcpyHostToDevice, s));
+  if (sens_snap && nb_ssnap) CU(cudaMemcpyAsync(dssnap.p, sens_snap, nb_ssnap, cudaMemcpyHostToDevice, s));
+  CU(cudaMemsetAsync(dq.p, 0, sizeof(int32_t), s));
+  CU(cudaMemcpyAsync(dst.p, stats, nb_stats, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dpm.p, params_pm, nb_pm, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dis.p, inv2sigma, nb_dir, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dat.p, atol_s, nb_dir, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dsens.p, sens, nb_sens, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(dsst.p, sens_stats, nb_sstats, cudaMemcpyHostToDevice, s));
+  DevProps props;
+  rc = current_props(props);
+  if (rc) return rc;
+  cudaError_t e = marlpde::launch_bdf_sens(dy.as<double>(), dp.as<marlpde_column_params>(), ds.as<marlpde_column_state>(),
+                                           n_columns, n_cells, *opts, dte.as<double>(), dsnap.as<double>(),
+                                           dst.as<int64_t>(), dec.as<int32_t>(), det.as<double>(), dw.as<double>(),
+                                           dq.as<int32_t>(), n_dirs, dpm.as<marlpde_column_params>(), dis.as<double>(),
+                                           dat.as<double>(), dsens.as<double>(), dssnap.as<double>(),
+                                           dsst.as<int64_t>(), dsw.as<double>(), props.sm_count, s);
+  if (e != cudaSuccess) return cuda_fail(e, "bdf sensitivity launch");
+  CU(cudaMemcpyAsync(y, dy.p, nb_y, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(state, ds.p, nb_s, cudaMemcpyDeviceToHost, s));
+  if (snapshots && nb_snap) CU(cudaMemcpyAsync(snapshots, dsnap.p, nb_snap, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(stats, dst.p, nb_stats, cudaMemcpyDeviceToHost, s));
+  if (event_counts) CU(cudaMemcpyAsync(event_counts, dec.p, nb_ec, cudaMemcpyDeviceToHost, s));
+  if (event_times && nb_et) CU(cudaMemcpyAsync(event_times, det.p, nb_et, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(sens, dsens.p, nb_sens, cudaMemcpyDeviceToHost, s));
+  if (sens_snap && nb_ssnap) CU(cudaMemcpyAsync(sens_snap, dssnap.p, nb_ssnap, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(sens_stats, dsst.p, nb_sstats, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  return MARLPDE_OK;
+}
+
 // ---- explicit Runge-Kutta integrators (RK23, DOP853): the implicit integrators' buffers and checks, no statistics ----
 static const char* erk_name(marlpde::ErkMethod m) { return m == marlpde::kErkRK23 ? "rk23" : "dop853"; }
 

@@ -206,13 +206,19 @@ def integrate_equations(solver_parms, tracker_parms, pde_parms):
     return field_solutions[:, :, -1], covered_time, depths, xstar, store_folder
 
 
-def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_folder=None, device=0):
+def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_folder=None, device=0, sensitivities=None):
     """Parameter sweep: `pde_parms` is a Map_Scenario dictionary whose values may be arrays of
     shape (B,) (see marlpde_b200.sweep_lattice) or a list of such dictionaries.  All columns are
     integrated in one launch of the kernel `method` selects (RK45: persistent on-chip kernel; RK23, DOP853: the batched
     explicit Runge-Kutta kernel; Radau, BDF / LSODA: the batched implicit kernels).  Returns the marlpde_b200.RK45Result / RadauResult;
     with `store_folder` one HDF5 file per sweep is written (datasets `solutions` (B,5,N,n_t),
-    `times`, `status`, `nfev`, `n_accepted`, `n_rejected`, `next_eval`, `t_reached`, `event_counts`)."""
+    `times`, `status`, `nfev`, `n_accepted`, `n_rejected`, `next_eval`, `t_reached`, `event_counts`).
+
+    `sensitivities` (methods BDF and LSODA only): a list of directions as for marlpde_b200.sensitivity_directions (each a
+    key of `pde_parms` or a {key: coefficient} dict), or the object that function returns.  The result then carries the
+    forward sensitivities dy/d eps at fixed nondimensional time (RadauResult.sensitivities / sens_y / sens_stats), and
+    the sweep file gains the dataset `sensitivities` (B, P, 5, N, n_t) and the attribute `sensitivity_directions`
+    (the direction names, one per line)."""
     if isinstance(pde_parms, (list, tuple)):
         keys = pde_parms[0].keys()
         pde_parms = {k: (np.array([p[k] for p in pde_parms]) if k != "N" else pde_parms[0]["N"]) for k in keys}
@@ -222,15 +228,22 @@ def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_fold
     if method not in ("RK45", "RK23", "DOP853", "Radau", "BDF", "LSODA"):
         raise NotImplementedError("the batched on-device integrators implement method='RK45', 'RK23', 'DOP853', 'Radau', "
                                   "'BDF' and 'LSODA' (the latter on the BDF kernel: LSODA's stiff mode)")
+    if sensitivities is not None and method not in ("BDF", "LSODA"):
+        raise NotImplementedError("forward sensitivities are implemented on the BDF kernel (methods 'BDF' and 'LSODA')")
     params = _mb.derive_column_params(pde_parms)
     y0 = _mb.initial_state(pde_parms)
+    extra = {}
+    if sensitivities is not None:
+        if not isinstance(sensitivities, _mb.SensitivityDirections):
+            sensitivities = _mb.sensitivity_directions(pde_parms, sensitivities)
+        extra = {"sensitivities": sensitivities}
     integrate = {"RK45": _mb.integrate_rk45_batch, "RK23": _mb.integrate_rk23_batch, "DOP853": _mb.integrate_dop853_batch,
                  "Radau": _mb.integrate_radau_batch}.get(method, _mb.integrate_bdf_batch)
     res = integrate(y0, params, t_span=solver_parms.get("t_span", (0, 1)),
                     first_step=solver_parms.get("first_step", 1e-6),
                     rtol=solver_parms.get("rtol", 1e-3), atol=solver_parms.get("atol", 1e-3),
                     max_step=solver_parms.get("max_step", np.inf), t_eval=tracker_parms["t_eval"],
-                    events=True, event_capacity=64, device=device)
+                    events=True, event_capacity=64, device=device, **extra)
     if store_folder is not None:
         os.makedirs(store_folder, exist_ok=True)
         with hdf5lite.File(os.path.join(store_folder, "LMAHeureuxPorosityDiff_sweep.hdf5"), "w") as stored:
@@ -242,6 +255,9 @@ def integrate_equations_batch(solver_parms, tracker_parms, pde_parms, store_fold
             stored.create_dataset("t_reached", data=res.t)
             for k in ("sedimentationrate", "b", "DCO3", "Xstar", "Tstar"):
                 stored.create_dataset("sweep_" + k, data=np.broadcast_to(np.asarray(pde_parms[k], float), res.t.shape))
+            if extra:
+                stored.create_dataset("sensitivities", data=np.transpose(np.asarray(res.sensitivities), (0, 1, 3, 4, 2)))
+                stored.attrs.update({"sensitivity_directions": "\n".join(sensitivities.names)})
             stored.attrs.update({k: v for k, v in (solver_parms | tracker_parms).items() if k != "jac_sparsity"})
     return res
 

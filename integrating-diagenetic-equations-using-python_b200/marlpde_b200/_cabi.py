@@ -102,6 +102,12 @@ SYMBOLS = {
                                         _P, _P, _P, _P, _P, C.c_int]),
     "marlpde_bdf_integrate_async": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
                                               _P, _P, _P, _P, _P, C.c_int, _P]),
+    "marlpde_bdf_sens_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "marlpde_bdf_sens_integrate_dev": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                                 _P, _P, _P, _P, _P, _P, C.c_size_t, _P, C.c_int,
+                                                 _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
+    "marlpde_bdf_sens_integrate": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
+                                             _P, _P, _P, _P, _P, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int]),
     "marlpde_rk23_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "marlpde_rk23_integrate_dev": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.POINTER(RK45Options),
                                              _P, _P, _P, _P, _P, C.c_size_t, _P, _P]),

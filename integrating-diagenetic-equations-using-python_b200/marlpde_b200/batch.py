@@ -264,6 +264,10 @@ class RadauResult:
     event_counts: np.ndarray = None   # [B,7]
     event_times: np.ndarray = None    # [B,7,capacity]
     state: np.ndarray = field(default=None, repr=False)
+    # forward sensitivities (integrate_bdf_batch(..., sensitivities=...)); None without them
+    sensitivities: object = None      # [B,P,n_eval,5,N] s = dy/d eps at t_eval (rows < next_eval are valid)
+    sens_y: object = None             # [B,P,5,N] s at the time reached (the w of a resumed call)
+    sens_stats: np.ndarray = None     # [B,3] corrector iterations, fallback factorisations, unconverged steps
 
     def solutions(self, column: int) -> np.ndarray:
         snap = self.snapshots[column]
@@ -297,21 +301,34 @@ def integrate_radau_batch(y0, params, t_span=(0.0, 1.0), first_step=1e-6, rtol=1
 def integrate_bdf_batch(y0, params, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e-3, t_eval=None,
                         max_step=np.inf, max_steps: int = 0, events: bool = False, event_capacity: int = 0,
                         state: np.ndarray | None = None, device: int = 0, inplace: bool = False,
-                          jac: str = "analytic") -> RadauResult:
+                          jac: str = "analytic", sensitivities=None, sens_y=None, sens_atol=None) -> RadauResult:
     """Implicit integration of every column with the variable-order BDF kernel (csrc/bdf_batch.cu): SciPy's `BDF`
     step for step (`solve_ivp(method="BDF", jac_sparsity=jacobian_sparsity())`, parameters.py:235-236) on the
     block-tridiagonal linear solver of the Radau kernel; also what `method="LSODA"` batches run on the device
     (parameters.py:214-219: LSODA is a BDF code on this stiff system).  Same result type as the Radau path; `nlu`
-    counts one real factorisation each.  A column resumed from `state` restarts at order 1."""
+    counts one real factorisation each.  A column resumed from `state` restarts at order 1.
+
+    `sensitivities` (a `marlpde_b200.sensitivity_directions(pde, wrt)` object for the same columns) adds forward
+    parameter sensitivities s_k = dy/d eps_k along each direction (staggered direct method, excluded from the error
+    control, DESIGN.md 5.4): the state's path is bit-identical to a run without them.  Derivatives are taken at fixed
+    nondimensional time t (a direction that moves Tstar gives dy(t)/d eps at fixed t, not at fixed years).  The result
+    then carries `sensitivities` [B,P,n_eval,5,N], `sens_y` [B,P,5,N] (s at the time reached) and `sens_stats` [B,3].
+    `sens_y` (default: the directions' w = dy0/d eps) is s at the start time — pass a budget-stopped result's `.sens_y`
+    back with its `.state` to resume; `sens_atol` [B,P] (default `sensitivities.atol(atol)`) is the absolute tolerance
+    of s in the corrector's convergence test."""
+    sens = None
+    if sensitivities is not None:
+        sens = (sensitivities, sensitivities.w if sens_y is None else sens_y,
+                sensitivities.atol(atol) if sens_atol is None else sens_atol)
     return _integrate_implicit("bdf", y0, params, t_span, first_step, rtol, atol, t_eval, max_step, max_steps, events,
-                               event_capacity, state, device, inplace, jac)
+                               event_capacity, state, device, inplace, jac, sens=sens)
 
 
 TEAM_AUTO_MAX_COLUMNS = 296     # 2 per SM: below this every column gets a two-warp team ("auto")
 
 
 def _integrate_implicit(kind, y0, params, t_span, first_step, rtol, atol, t_eval, max_step, max_steps, events,
-                        event_capacity, state, device, inplace, jac="analytic", team_columns=0) -> RadauResult:
+                        event_capacity, state, device, inplace, jac="analytic", team_columns=0, sens=None) -> RadauResult:
     """`jac`: "analytic" (default) — every 5x5 block analytic in one pass, no RHS evaluations; only for a cell that sits ON
     a switching surface of the model the porosity column is num_jac's one-sided difference (csrc/implicit_common.cuh);
     "fd" (MARLPDE_FLAG_JAC_FD) — analytic off-diagonal blocks, diagonal blocks by finite differences with num_jac's step
@@ -375,10 +392,29 @@ def _integrate_implicit(kind, y0, params, t_span, first_step, rtol, atol, t_eval
             nb = int(f_ws(B, N))
             d_work = torch.empty(max(nb, 8) // 8, dtype=torch.float64, device=dev)
             stream = torch.cuda.current_stream().cuda_stream
-            _cabi.check(f_dev(
-                y.data_ptr(), d_params.data_ptr(), d_state.data_ptr(), B, N, C.byref(opts),
-                d_te.data_ptr() if n_eval else None, d_snap.data_ptr(), d_ec.data_ptr(), d_et.data_ptr(),
-                d_stats.data_ptr(), d_work.data_ptr(), nb, d_queue.data_ptr(), stream))
+            if sens is None:
+                _cabi.check(f_dev(
+                    y.data_ptr(), d_params.data_ptr(), d_state.data_ptr(), B, N, C.byref(opts),
+                    d_te.data_ptr() if n_eval else None, d_snap.data_ptr(), d_ec.data_ptr(), d_et.data_ptr(),
+                    d_stats.data_ptr(), d_work.data_ptr(), nb, d_queue.data_ptr(), stream))
+            else:
+                sd, sy, sat = _sens_inputs(sens, B, N)
+                P = sd.n_dirs
+                d_pm = torch.from_numpy(sd.params_pm.view(np.uint8).reshape(-1).copy()).to(dev)
+                d_i2s = torch.from_numpy(sd.inv2sigma.copy()).to(dev)
+                d_sat = torch.from_numpy(sat.copy()).to(dev)
+                d_sens = (sy.clone() if _is_torch(sy) else torch.from_numpy(np.array(sy)).to(dev)).contiguous()
+                d_ssnap = torch.full((B, P, n_eval, 5, N), float("nan"), dtype=torch.float64, device=dev)
+                d_sstats = torch.zeros((B, 3), dtype=torch.int64, device=dev)
+                nbs = int(lib.marlpde_bdf_sens_workspace_bytes(B, N, P))
+                d_swork = torch.empty(max(nbs, 8) // 8, dtype=torch.float64, device=dev)
+                _cabi.check(lib.marlpde_bdf_sens_integrate_dev(
+                    y.data_ptr(), d_params.data_ptr(), d_state.data_ptr(), B, N, C.byref(opts),
+                    d_te.data_ptr() if n_eval else None, d_snap.data_ptr(), d_ec.data_ptr(), d_et.data_ptr(),
+                    d_stats.data_ptr(), d_work.data_ptr(), nb, d_queue.data_ptr(), P, d_pm.data_ptr(),
+                    d_i2s.data_ptr(), d_sat.data_ptr(), d_sens.data_ptr(), d_ssnap.data_ptr(), d_sstats.data_ptr(),
+                    d_swork.data_ptr(), nbs, stream))
+                sens_out = (d_ssnap, d_sens, d_sstats.cpu().numpy())
             st_out = d_state.cpu().numpy().view(STATE_DTYPE).reshape(B)
             stats = d_stats.cpu().numpy()
             ec, et = d_ec.cpu().numpy(), d_et.cpu().numpy()[:, :, :cap]
@@ -394,16 +430,45 @@ def _integrate_implicit(kind, y0, params, t_span, first_step, rtol, atol, t_eval
         stats = np.zeros((B, 4), dtype=np.int64)
         ec = np.zeros((B, NEVENTS), dtype=np.int32)
         et = np.full((B, NEVENTS, cap), np.nan)
-        _cabi.check(f_host(
-            _cabi.ptr(y), _cabi.ptr(p), _cabi.ptr(st_out), B, N, C.byref(opts),
-            _cabi.ptr(t_eval_arr) if n_eval else None, _cabi.ptr(snaps) if n_eval else None, _cabi.ptr(ec),
-            _cabi.ptr(et) if cap else None, _cabi.ptr(stats), device))
+        if sens is None:
+            _cabi.check(f_host(
+                _cabi.ptr(y), _cabi.ptr(p), _cabi.ptr(st_out), B, N, C.byref(opts),
+                _cabi.ptr(t_eval_arr) if n_eval else None, _cabi.ptr(snaps) if n_eval else None, _cabi.ptr(ec),
+                _cabi.ptr(et) if cap else None, _cabi.ptr(stats), device))
+        else:
+            sd, sy, sat = _sens_inputs(sens, B, N)
+            P = sd.n_dirs
+            s_y = np.array(sy.cpu().numpy() if _is_torch(sy) else sy, dtype=np.float64, order="C", copy=True)
+            s_snap = np.full((B, P, n_eval, 5, N), np.nan)
+            s_stats = np.zeros((B, 3), dtype=np.int64)
+            _cabi.check(lib.marlpde_bdf_sens_integrate(
+                _cabi.ptr(y), _cabi.ptr(p), _cabi.ptr(st_out), B, N, C.byref(opts),
+                _cabi.ptr(t_eval_arr) if n_eval else None, _cabi.ptr(snaps) if n_eval else None, _cabi.ptr(ec),
+                _cabi.ptr(et) if cap else None, _cabi.ptr(stats), P, _cabi.ptr(sd.params_pm), _cabi.ptr(sd.inv2sigma),
+                _cabi.ptr(sat), _cabi.ptr(s_y), _cabi.ptr(s_snap) if n_eval else None, _cabi.ptr(s_stats), device))
+            sens_out = (s_snap, s_y, s_stats)
+    extra = {} if sens is None else dict(sensitivities=sens_out[0], sens_y=sens_out[1], sens_stats=sens_out[2])
     return RadauResult(y=y, t=st_out["t"].copy(), h_abs=st_out["h_abs"].copy(), status=st_out["status"].copy(),
                        n_accepted=st_out["n_accepted"].copy(), n_rejected=st_out["n_rejected"].copy(),
                        nfev=st_out["nfev"].copy(), njev=stats[:, 0].copy(), nlu=stats[:, 1].copy(),
                        newton_iterations=stats[:, 2].copy(), newton_failures=stats[:, 3].copy(),
                        t_eval=t_eval_arr, snapshots=snaps, next_eval=st_out["next_eval"].copy(), event_counts=ec,
-                       event_times=et, state=st_out)
+                       event_times=et, state=st_out, **extra)
+
+
+def _sens_inputs(sens, B, N):
+    """Checked (directions, s at the start time [B,P,5,N], atol_s [B,P]) of a sensitivity run."""
+    sd, sy, sat = sens
+    P = sd.n_dirs
+    if sd.params_pm.shape != (B, P, 2) or sd.w.shape != (B, P, 5, N):
+        raise ValueError(f"sensitivity directions were derived for {sd.params_pm.shape[0]} columns of "
+                         f"{sd.w.shape[-1]} cells, the batch has {B} of {N}")
+    if tuple(sy.shape) != (B, P, 5, N):
+        raise ValueError(f"sens_y must have shape {(B, P, 5, N)}; got {tuple(sy.shape)}")
+    sat = np.ascontiguousarray(np.broadcast_to(np.asarray(sat, dtype=np.float64), (B, P)))
+    if np.any(~(sat > 0)):
+        raise ValueError("sens_atol must be positive")
+    return sd, sy, sat
 
 
 def integrate_rk23_batch(y0, params, t_span=(0.0, 1.0), first_step=1e-6, rtol=1e-3, atol=1e-3, t_eval=None,
